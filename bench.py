@@ -13,6 +13,8 @@ configurations: NovaSeq-shaped 150 bp in the native format, PacBio-shaped long r
 among 4 + 4 models), `e2e_file` (FASTQ text -> .idn -> FASTQ text through the host mirror of the reference API, with and
 without identifiers, and the identifiers codec alone), `fastq_text`, `other_mode` and, at N > 1, `strong_scaling` (ONE file
 over the ranks).  --no-extra-workloads / --no-e2e / --no-fastq / --no-other-mode / --no-cpu-baseline trim the run.
+--dump-outputs DIR writes what the last timed step of the headline workload handed back as DIR/<name>.npy (see
+dump_outputs), so that two builds run with the same arguments can be compared output for output.
 Nothing here reads /root/reference.
 The oracle (oracle/) is used only for `cpu_baseline` / `--impl reference`: the Rust reference cannot be built in
 this image, so its CPU restatement (pinned bit-exactly to the reference's golden container) is what is timed.
@@ -335,6 +337,62 @@ def retained_models(env, w: dict, block_reads: int):
     return names
 
 
+DUMP_SEED = 20240604
+DUMP_SAMPLES = {"container": 4 << 20, "symbols": 2 << 20, "reads": 1 << 20}  # 40 MiB of samples at most
+
+
+def _sample_positions(rng, n: int, k: int) -> np.ndarray:
+    """k seeded positions in [0, n), ascending; all of them when n <= k"""
+    return np.arange(n, dtype=np.int64) if n <= k else np.sort(rng.integers(0, n, size=k, dtype=np.int64))
+
+
+def dump_outputs(out_dir: Path, chunks, out_d, dec_a, dec_q, S: int):
+    """What the compress and decompress calls of the last timed step returned, as DIR/<name>.npy in float32 / float64
+    (exact for bytes, CRCs and offsets below 2^53).  The whole outputs run to gigabytes, so the per-block tables are
+    complete and the byte arrays are seeded samples (positions drawn from DUMP_SEED and the output's length):
+      block_offsets       float64 [blocks + 1]  offset of every block in the concatenated container
+      block_crc           float64 [blocks]      the CRC-32 the compressor returned for every block
+      block_bytes_crc32   float64 [blocks]      CRC-32 of every block's container bytes (covers all of them)
+      container_sample    float32               container bytes at sampled positions
+      acids_sample        float32               decoded acids at sampled symbol positions
+      quals_sample        float32               decoded quality scores at the same positions
+      read_off_sample     float64               decoded read offsets at sampled read indices"""
+    import zlib
+    import torch
+    rng = np.random.Generator(np.random.PCG64(DUMP_SEED))
+    offs, crcs, digests, samples = [np.zeros(1, dtype=np.int64)], [], [], []
+    base = 0
+    block_off = [c.block_off.cpu().numpy() for c in chunks]
+    total = sum(int(b[-1]) for b in block_off)
+    pos = _sample_positions(rng, total, DUMP_SAMPLES["container"])
+    for c, boff in zip(chunks, block_off):
+        n = int(boff[-1])
+        data = out_d[c.out_base:c.out_base + n].cpu().numpy()
+        offs.append(base + boff[1:])
+        crcs.append(c.block_crc.cpu().numpy().view(np.uint32))
+        digests += [zlib.crc32(data[int(boff[b]):int(boff[b + 1])]) for b in range(c.n_blocks)]
+        lo, hi = np.searchsorted(pos, [base, base + n])
+        samples.append(data[pos[lo:hi] - base])
+        base += n
+    sym = torch.from_numpy(_sample_positions(rng, S, DUMP_SAMPLES["symbols"])).to(dec_a.device)
+    read_off = torch.cat([c.dec_read_off[:-1] + c.s0 for c in chunks] + [torch.tensor([S], device=dec_a.device)])
+    ridx = torch.from_numpy(_sample_positions(rng, len(read_off), DUMP_SAMPLES["reads"])).to(dec_a.device)
+    arrays = {
+        "block_offsets": np.concatenate(offs).astype(np.float64),
+        "block_crc": np.concatenate(crcs).astype(np.float64),
+        "block_bytes_crc32": np.asarray(digests, dtype=np.float64),
+        "container_sample": np.concatenate(samples).astype(np.float32),
+        "acids_sample": dec_a[sym].cpu().numpy().astype(np.float32),
+        "quals_sample": dec_q[sym].cpu().numpy().astype(np.float32),
+        "read_off_sample": read_off[ridx].cpu().numpy().astype(np.float64),
+    }
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(out_dir / f"{k}.npy", v)
+    print(f"bench: {len(arrays)} output arrays ({sum(v.nbytes for v in arrays.values()) / 2**20:.1f} MiB) written to {out_dir}",
+          file=sys.stderr)
+
+
 def run_workload(env, args, name: str, w: dict, *, steps: int, warmup: int, main: bool, shard=None, no_e2e=False, after=None):
     """One workload on this rank's GPU: device-resident leg (timed with CUDA events), optional e2e leg (host buffers),
     and for the main workload the FASTQ text leg.  Returns the raw numbers of this rank; run_gpu reduces them over ranks."""
@@ -355,6 +413,8 @@ def run_workload(env, args, name: str, w: dict, *, steps: int, warmup: int, main
         # ~1 more for the library's workspaces of a 1024-block call and the e2e staging
         free_b, _ = torch.cuda.mem_get_info()
         fit = int(0.80 * free_b / (6.5 * (lo + hi) / 2))
+        if n_reads > fit and main and args.dump_outputs:  # a dump is only comparable with one of the same inputs
+            raise SystemExit(f"{n_reads} reads asked, {fit} fit the free device memory: pass --reads to dump a fixed workload")
         if n_reads > fit:
             note = f"{n_reads} reads asked, {fit} fit the free device memory ({free_b / 1e9:.0f} GB)"
             n_reads = fit
@@ -523,6 +583,8 @@ def run_workload(env, args, name: str, w: dict, *, steps: int, warmup: int, main
     elif not main and world == 1 and main_mode == "native" and not args.no_other_mode:
         other = measure(other_mode, 1, 3, False)  # the ratio delta against the compat output on the same input (north_star)
     m = measure(main_mode, steps, warmup, True)
+    if main and args.dump_outputs and rank == 0:  # before the legs below reuse the device buffers
+        dump_outputs(Path(args.dump_outputs), chunks, out_d, dec_a, dec_q, S)
 
     fastq = None
     e2e_file = None
@@ -1158,7 +1220,13 @@ def main():
     ap.add_argument("--text-chunk-mb", type=int, default=256, help="FASTQ text per device call of that leg")
     ap.add_argument("--file-batch-blocks", type=int, default=32, help="blocks per batch in the e2e_file decode (and in add_batch)")
     ap.add_argument("--e2e-profile", action="store_true", help="print the host-side phase times of the e2e leg to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step of the headline workload to DIR/<name>.npy (GPU arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.warmup < 3:
         args.warmup = 3
     w = dict(WORKLOADS[args.workload])
