@@ -1,4 +1,6 @@
-"""Helpers shared by the parity tests: feed oracle-side model data through the C-ABI; synthetic models per spec type."""
+"""Helpers shared by the parity tests: feed oracle-side model data through the C-ABI; synthetic models per spec type;
+the bundled same-sequencer model pairs and model-driven reads drawn on the device."""
+import ctypes as C
 import re
 
 import numpy as np
@@ -85,3 +87,31 @@ def synthetic_model(O, mtype, spec_name, reads, seed, n_ctx=3):
     return O.Model(O.ModelData.from_contexts(mtype, spec_name, ctxs))
 
 
+# (acid model, q-score model, read lengths, expected kernel variant): the same-sequencer pairs of models/ (models.md)
+PAIRS = {
+    "hiseq2000": ("ERR174310__human__illumina_hiseq_2000__acids", "SRR2962693__human__illumina_hiseq_2500__q_scores", (100, 100), 0),
+    "hiseq2500_human": ("SRR2962693__human__illumina_hiseq_2500__acids", "SRR2962693__human__illumina_hiseq_2500__q_scores", (70, 101), 0),
+    "hiseq2500_b_stabilis": ("SRR19549058__b_stabilis__illumina_hiseq_2500__acids", "SRR19549058__b_stabilis__illumina_hiseq_2500__q_scores", (125, 125), 0),
+    "novaseq_human": ("SRR8861483__human__illumina_novaseq_6000__acids", "SRR8861483__human__illumina_novaseq_6000__q_scores", (150, 150), 1),
+    "sequel2": ("m64187e__sars_cov_2__sequel_ii_e__acids", "m64187e__sars_cov_2__sequel_ii_e__q_scores", (10_000, 20_000), 2),
+    "novaseq_cat": ("SRR18908372__cat__illumina_novaseq_6000__acids", "SRR18908372__cat__illumina_novaseq_6000__q_scores", (151, 151), 3),
+    "hiseq2500_cat": ("SRR5373739__cat__illumina_hiseq_2500__acids", "SRR5373739__cat__illumina_hiseq_2500__q_scores", (90, 126), 4),
+    "iseq100": ("ERR5462922__ebov__illumina_iseq_100__acids", "ERR5462922__ebov__illumina_iseq_100__q_scores", (151, 151), 5),
+    "hiseq2500_e_coli": ("SRR16141966__e_coli__illumina_hiseq_2500__acids", "SRR16141966__e_coli__illumina_hiseq_2500__q_scores", (100, 100), 6),
+    "hiseq2500_pear": ("SRR19609907__pear__illumina_hiseq_2500__acids", "SRR19609907__pear__illumina_hiseq_2500__q_scores", (101, 101), 7),
+    "hiseq2500_salmonella": ("SRR20210997__salmonella__illumina_hiseq_2500__acids", "SRR20210997__salmonella__illumina_hiseq_2500__q_scores", (100, 100), -1),
+}
+
+
+def synth_on_device(gctx, ha, hq, read_off, seed, n_ppm=500):
+    """Model-driven reads (idn_gpu_synth_reads_dev; equal to the oracle's sampler, test_gpu_parity.py) -> host arrays."""
+    import torch
+    S = int(read_off[-1])
+    ro_d = torch.from_numpy(read_off.view(np.int64)).cuda()
+    a_d = torch.zeros(S + 16, dtype=torch.uint8, device="cuda")
+    q_d = torch.zeros(S + 16, dtype=torch.uint8, device="cuda")
+    sp = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    gctx.check(gctx.L.idn_gpu_synth_reads_dev(gctx.h, ha, hq, ro_d.data_ptr(), len(read_off) - 1, 0, seed, n_ppm,
+                                              a_d.data_ptr(), q_d.data_ptr(), sp))
+    torch.cuda.synchronize()
+    return a_d[:S].cpu().numpy(), q_d[:S].cpu().numpy()
