@@ -357,7 +357,9 @@ class Context:
         n = int(ro[-1]) if reads_cap else 0
         return ro, a[:n], q[:n]
 
-    def decompress_reads(self, payload, pay_off, pay_len, seq_len, acid_model, q_model, models):
+    def decompress_reads(self, payload, pay_off, pay_len, seq_len, acid_model, q_model, models, out_off=None):
+        """Decode reads from their payloads (idn_read_index).  out_off defaults to the exclusive scan of seq_len.  On error
+        the raised IdnGpuError carries .read_status (the per-read status the kernel wrote; zeros if it never ran)."""
         payload = _c(payload, np.uint8)
         po = _c(pay_off, np.uint64)
         pl = _c(pay_len, np.uint32)
@@ -365,15 +367,22 @@ class Context:
         am = _c(acid_model, np.uint8)
         qm = _c(q_model, np.uint8)
         m = _c(models, np.int32)
-        oo = np.zeros(len(sl) + 1, dtype=np.uint64)
-        np.cumsum(sl, out=oo[1:])
+        if out_off is None:
+            oo = np.zeros(len(sl) + 1, dtype=np.uint64)
+            np.cumsum(sl, out=oo[1:])
+        else:
+            oo = _c(out_off, np.uint64)
         idx = ReadIndex(len(sl), _p(po), _p(pl), _p(sl), oo.ctypes.data, _p(am), _p(qm))
-        S = int(oo[-1])
+        S = int(sl.sum(dtype=np.uint64))
         a = np.zeros(max(S, 1), dtype=np.uint8)
         q = np.zeros(max(S, 1), dtype=np.uint8)
         st = np.zeros(max(len(sl), 1), dtype=np.uint32)
-        self.check(self.L.idn_gpu_decompress_reads(self.h, _p(payload), payload.size, C.byref(idx), _p(m), len(m),
-                                                   a.ctypes.data, q.ctypes.data, st.ctypes.data))
+        rc = self.L.idn_gpu_decompress_reads(self.h, _p(payload), payload.size, C.byref(idx), _p(m), len(m),
+                                             a.ctypes.data, q.ctypes.data, st.ctypes.data)
+        if rc != OK:
+            e = IdnGpuError(rc, self.L.idn_gpu_last_error(self.h).decode())
+            e.read_status = st[:len(sl)]
+            raise e
         return oo, a[:S], q[:S], st[:len(sl)]
 
     def block_crc(self, read_off, acids, quals, block_first_read, name_off=None, names=None) -> np.ndarray:

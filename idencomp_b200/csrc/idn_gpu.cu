@@ -1961,7 +1961,8 @@ extern "C" int32_t idn_gpu_decompress_reads(idn_gpu_ctx* ctx, const uint8_t* pay
     if (!payload && payload_bytes) return fail(ctx, IDN_E_INVALID_ARG, "payload is NULL");
     uint64_t S = 0;
     for (uint64_t r = 0; r < R; r++) {
-        if (index->pay_off[r] + index->pay_len[r] > payload_bytes) return fail(ctx, IDN_E_SERIALIZE, "read %llu payload out of range", (unsigned long long)r);
+        // (not pay_off + pay_len > payload_bytes: that sum wraps for an offset near 2^64)
+        if (index->pay_len[r] > payload_bytes || index->pay_off[r] > payload_bytes - index->pay_len[r]) return fail(ctx, IDN_E_SERIALIZE, "read %llu payload out of range", (unsigned long long)r);
         if (index->out_off[r] != S) return fail(ctx, IDN_E_INVALID_ARG, "out_off is not the exclusive scan of seq_len");
         S += index->seq_len[r];
         if (index->acid_model[r] >= n_models || index->q_model[r] >= n_models)

@@ -103,6 +103,47 @@ PAIRS = {
 }
 
 
+def parse_compat_block(data: bytes, is_acid, offsets=False):
+    """Walk the slices of one compat block: 00 Identifiers (u32be len, u8 codec, data), 01 SwitchModel (u8 index),
+    02 Sequence (u32be len, u32be seq_len, payload) (data.rs:46-84).  is_acid[i]: container model i is an acid model.
+    -> (acid index, q-score index, acid switch before the read, q-score switch before the read), one entry per read;
+    with offsets=True also (payload offset in `data`, payload length, sequence length) per read."""
+    u32 = lambda pos: int.from_bytes(data[pos:pos + 4], "big")
+    acid, qual, sw_a, sw_q, p_off, p_len, s_len = [], [], [], [], [], [], []
+    cur_a = cur_q = -1
+    pend_a = pend_q = False
+    pos, n = 0, len(data)
+    while pos < n:
+        kind = data[pos]
+        if kind == 0:
+            pos += 6 + u32(pos + 1)
+        elif kind == 1:
+            idx = data[pos + 1]
+            if is_acid[idx]:
+                cur_a, pend_a = idx, True
+            else:
+                cur_q, pend_q = idx, True
+            pos += 2
+        elif kind == 2:
+            acid.append(cur_a)
+            qual.append(cur_q)
+            sw_a.append(pend_a)
+            sw_q.append(pend_q)
+            pend_a = pend_q = False
+            p_off.append(pos + 9)
+            p_len.append(u32(pos + 1))
+            s_len.append(u32(pos + 5))
+            pos += 9 + u32(pos + 1)
+        else:
+            raise ValueError(f"unknown slice kind {kind} at byte {pos}")
+    if pos != n:
+        raise ValueError("the last slice overruns the block")
+    out = (np.asarray(acid), np.asarray(qual), np.asarray(sw_a, dtype=bool), np.asarray(sw_q, dtype=bool))
+    if offsets:
+        out += (np.asarray(p_off, dtype=np.uint64), np.asarray(p_len, dtype=np.uint32), np.asarray(s_len, dtype=np.uint32))
+    return out
+
+
 def synth_on_device(gctx, ha, hq, read_off, seed, n_ppm=500):
     """Model-driven reads (idn_gpu_synth_reads_dev; equal to the oracle's sampler, test_gpu_parity.py) -> host arrays."""
     import torch

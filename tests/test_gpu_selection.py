@@ -29,7 +29,7 @@ import numpy as np
 import pytest
 
 from conftest import MODELS, ROOT
-from gpu_util import PAIRS, SPEC_NAMES, blocks_of, synth_on_device, synthetic_model, toy_reads, upload
+from gpu_util import PAIRS, SPEC_NAMES, blocks_of, parse_compat_block, synth_on_device, synthetic_model, toy_reads, upload
 
 COMPAT, NATIVE = 1, 2
 BLOCK = 4 * 1024 * 1024
@@ -64,39 +64,6 @@ def split_container(idn: bytes):
         pos += ln
     assert pos == len(idn)
     return idn[8], ids, blocks
-
-
-def parse_compat_block(data: bytes, is_acid):
-    """Walk the slices of one compat block: 00 Identifiers (u32be len, u8 codec, data), 01 SwitchModel (u8 index),
-    02 Sequence (u32be len, u32be seq_len, payload) (data.rs:46-84).  is_acid[i]: container model i is an acid model.
-    -> (acid index, q-score index, acid switch before the read, q-score switch before the read), one entry per read."""
-    acid, qual, sw_a, sw_q = [], [], [], []
-    cur_a = cur_q = -1
-    pend_a = pend_q = False
-    pos, n = 0, len(data)
-    while pos < n:
-        kind = data[pos]
-        if kind == 0:
-            pos += 6 + _u32(data, pos + 1)
-        elif kind == 1:
-            idx = data[pos + 1]
-            if is_acid[idx]:
-                cur_a, pend_a = idx, True
-            else:
-                cur_q, pend_q = idx, True
-            pos += 2
-        elif kind == 2:
-            acid.append(cur_a)
-            qual.append(cur_q)
-            sw_a.append(pend_a)
-            sw_q.append(pend_q)
-            pend_a = pend_q = False
-            pos += 9 + _u32(data, pos + 1)
-        else:
-            raise ValueError(f"unknown slice kind {kind} at byte {pos}")
-    if pos != n:
-        raise ValueError("the last slice overruns the block")
-    return np.asarray(acid), np.asarray(qual), np.asarray(sw_a, dtype=bool), np.asarray(sw_q, dtype=bool)
 
 
 def native_lane_models(data: bytes):
