@@ -117,7 +117,7 @@ struct idn_gpu_ctx {
     int32_t walk_mode = 0;  // idn_gpu_set_walk
     uint32_t* d_crc_tab = nullptr;  // [256]
     uint32_t* d_xpow = nullptr;     // [64]
-    uint32_t* d_crc_back = nullptr;  // [512 + 2 * kCrcLenTab]: Tinv | U (backward CRC step) | {x^(8n), x^(16n)} for n < kCrcLenTab
+    uint32_t* d_crc_back = nullptr;  // [256 + 2 * kCrcLenTab]: Tinv (backward CRC step) | {x^(8n), x^(16n)} for n < kCrcLenTab
     bool enc_crc = true;             // IDN_NO_ENC_CRC=1: the per-read CRC partials of a compress call come from crc_read_kernel
     // workspaces of the *_dev paths
     DevBuf w_scratch, w_paylen, w_sizes, w_chosen, w_tiles, w_sliceoff, w_readblock, w_small, w_crcpart, w_crclen;
@@ -377,15 +377,12 @@ static void make_crc_tables(uint32_t* tab, uint32_t* xpow) {
 }
 
 // Tables of the backward CRC the encoder runs (it visits a read's symbols last to first; EncCrc in idn_kernels.cuh):
-// Tinv / U undo one "advance by a zero byte" step, xlen[n] = {x^(8n), x^(16n)} mod P bring the result back into place.
-static void make_crc_back_tables(const uint32_t* tab, const uint32_t* xpow, uint32_t* back /*[512 + 2 * kCrcLenTab]*/) {
+// Tinv undoes one "advance by a zero byte" step, xlen[n] = {x^(8n), x^(16n)} mod P bring the result back into place.
+static void make_crc_back_tables(const uint32_t* tab, const uint32_t* xpow, uint32_t* back /*[256 + 2 * kCrcLenTab]*/) {
     uint32_t rtop[256];
     for (uint32_t i = 0; i < 256; i++) rtop[tab[i] >> 24] = i;  // the top bytes of the table are a permutation
     uint32_t* tinv = back;
-    uint32_t* u = back + 256;
     for (uint32_t t = 0; t < 256; t++) tinv[t] = (tab[rtop[t]] << 8) | rtop[t];
-    auto linv = [&](uint32_t v) { return (v << 8) ^ tinv[v >> 24]; };
-    for (uint32_t b = 0; b < 256; b++) u[b] = linv(tab[b]);
     auto mul = [](uint32_t a, uint32_t b) {
         uint32_t p = 0;
         for (int i = 0; i < 32; i++) {
@@ -395,7 +392,7 @@ static void make_crc_back_tables(const uint32_t* tab, const uint32_t* xpow, uint
         }
         return p;
     };
-    uint32_t* xlen = back + 512;
+    uint32_t* xlen = back + 256;
     uint32_t x = 0x80000000u;  // x^0
     for (uint32_t n = 0; n < kCrcLenTab; n++) {
         xlen[2 * n] = x;
@@ -435,7 +432,7 @@ extern "C" int32_t idn_gpu_create(int32_t device, idn_gpu_ctx** out) {
     if (cudaMemcpy(ctx->d_crc_tab, tab, sizeof tab, cudaMemcpyHostToDevice) != cudaSuccess) return bail("cudaMemcpy");
     if (cudaMemcpy(ctx->d_xpow, xpow, sizeof xpow, cudaMemcpyHostToDevice) != cudaSuccess) return bail("cudaMemcpy");
     {
-        std::vector<uint32_t> back(512 + 2 * kCrcLenTab);
+        std::vector<uint32_t> back(256 + 2 * kCrcLenTab);
         make_crc_back_tables(tab, xpow, back.data());
         if (cudaMalloc(&ctx->d_crc_back, back.size() * 4) != cudaSuccess) return bail("cudaMalloc");
         if (cudaMemcpy(ctx->d_crc_back, back.data(), back.size() * 4, cudaMemcpyHostToDevice) != cudaSuccess) return bail("cudaMemcpy");

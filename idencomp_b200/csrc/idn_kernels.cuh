@@ -138,6 +138,22 @@ struct SymBackReader {
         left--;
         if ((left & 3) == 0 && left != 0) next_word();
     }
+    // vec only, at a word boundary ((left & 3) == 0): the next four bytes in ca / cq (first one in bits 24..31), taken
+    // by the caller before it calls skip_word().  The caller guarantees that their chunk lies inside the arrays (above it
+    // lies the chunk already read, so only its lower end is in question).
+    __device__ __forceinline__ void peek_word() {
+        if (left == 0) {
+            const uint4 va = __ldg(reinterpret_cast<const uint4*>(c)), vq = __ldg(reinterpret_cast<const uint4*>(qbase + (c - abase)));
+            ca = va.w; a2 = va.z; a1 = va.y; a0 = va.x;
+            cq = vq.w; q2 = vq.z; q1 = vq.y; q0 = vq.x;
+            c -= 16;
+            left = 16;
+        }
+    }
+    __device__ __forceinline__ void skip_word() {
+        left -= 4;
+        next_word();  // (when left reaches 0 the next peek_word() reloads all of them)
+    }
 };
 
 // writes bytes at decreasing addresses, 4 at a time.  `end` must be 4-byte aligned.  Bytes wait in a 64-bit
@@ -391,7 +407,7 @@ struct EncodeArgs {
     const uint8_t* switched;            // [2][n_reads]: a SwitchModel slice precedes the read's Sequence slice, or nullptr
     const uint8_t* cand_index;          // [2][kMaxCand] candidate -> SwitchModel index
     // optional: the per-read CRC-32 partials crc(acids | quals) for crc_block_kernel, computed on the way (EncCrc)
-    const uint32_t* crc_back;           // [512 + 2 * kCrcLenTab] (make_crc_back_tables), or nullptr
+    const uint32_t* crc_back;           // [256 + 2 * kCrcLenTab] (make_crc_back_tables), or nullptr
     const uint32_t* xpow;               // [64]
     uint32_t* part_crc;
     unsigned long long* part_len;
@@ -431,19 +447,29 @@ struct EncStream {
 // CRC-32 of a byte string whose bytes arrive LAST TO FIRST (the encoder's order).  With L = "advance the register by one
 // zero byte" (c -> tab[c & 0xff] ^ (c >> 8), linear over GF(2)) the register after the string b_0 .. b_{n-1} is
 // L^n(ff..f) ^ XOR_i L^(n-1-i)(tab[b_i]).  Keeping B = L^-(n-i)(contribution of b_i .. b_{n-1}) turns the backward walk into
-// B <- Linv(B) ^ Linv(tab[b]) = (B << 8) ^ tinv[B >> 24] ^ u[b]  -- one shift and two look-ups per byte, like the forward
-// step -- and crc = ~L^n(B ^ ff..f), where L^n is the multiplication by x^(8n) mod P (gf2_mul).  For acids | quals of one
-// read (two strings of n bytes walked in lock step): crc = ~(x^(8n) * Bq  ^  x^(16n) * (Ba ^ ff..f)).
+// B <- Linv(B) ^ Linv(tab[b]) = (B << 8) ^ tinv[B >> 24] ^ b  -- tab[b] = L(b), so Linv(tab[b]) is the byte itself: one
+// shift and one look-up per byte -- and crc = ~L^n(B ^ ff..f), where L^n is the multiplication by x^(8n) mod P (gf2_mul).
+// Linv(v) = v << 8 for v < 2^24 (tinv[0] = 0), so four bytes w = b_i b_{i+1} b_{i+2} b_{i+3} (b_i in bits 24..31) step
+// B <- Linv^4(B) ^ w.  For acids | quals of one read (two strings of n bytes walked in lock step):
+// crc = ~(x^(8n) * Bq  ^  x^(16n) * (Ba ^ ff..f)).
 constexpr uint32_t kCrcLenTab = 1024;  // read lengths whose x^(8n), x^(16n) come from a table
 __device__ __forceinline__ uint32_t gf2_mul(uint32_t a, uint32_t b);  // (K7 section below)
 __device__ __forceinline__ uint32_t x8n_mod_p(unsigned long long n, const uint32_t* __restrict__ xpow);
 struct EncCrc {
     const uint32_t* tinv;  // shared memory [256], or nullptr: no CRC
-    const uint32_t* u;     // shared memory [256]
     uint32_t ba, bq;
     __device__ __forceinline__ void add(uint32_t a, uint32_t q) {
-        ba = (ba << 8) ^ tinv[ba >> 24] ^ u[a];
-        bq = (bq << 8) ^ tinv[bq >> 24] ^ u[q];
+        ba = (ba << 8) ^ tinv[ba >> 24] ^ a;
+        bq = (bq << 8) ^ tinv[bq >> 24] ^ q;
+    }
+    __device__ __forceinline__ void add_word(uint32_t wa, uint32_t wq) {
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            ba = (ba << 8) ^ tinv[ba >> 24];
+            bq = (bq << 8) ^ tinv[bq >> 24];
+        }
+        ba ^= wa;
+        bq ^= wq;
     }
 };
 
@@ -474,10 +500,17 @@ __device__ __forceinline__ void encode_read_body(const ModelDev& ma, const Model
     GenBack ga, gq;
     ga.clear(sa);
     gq.clear(sq);
-    int32_t front = (int32_t)p1 - 1;  // next position to pull into the windows (reads are shorter than 2^31)
-    uint32_t raw_a = 0;                // raw symbols travel in two more shift registers (entry k = position j - k)
+    uint32_t raw_a = 0;  // raw symbols travel in two more shift registers (entry k = position j - k)
     unsigned long long raw_q = 0;
-    auto pull = [&]() {
+    auto shift_in = [&](uint32_t a, uint32_t q) {
+        const bool z = a * q == 0;
+        ga.shift_in(sa, a, q, z);
+        gq.shift_in(sq, a, q, z);
+        raw_a = (raw_a >> 3) | (a << (3 * kHist));
+        raw_q = (raw_q >> 7) | ((unsigned long long)q << (7 * kHist));
+    };
+    // pulls position `front` into the windows (zeros in front of the read: front < 0); called for p1-1, p1-2, ... in turn
+    auto pull = [&](int32_t front) {
         uint32_t a = 0, q = 0;
         if (front >= 0) {
 #ifndef IDN_NO_SYM16
@@ -493,15 +526,10 @@ __device__ __forceinline__ void encode_read_body(const ModelDev& ma, const Model
             }
             if (C.tinv) C.add(a, q);  // uniform per launch; whole reads only (every position is pulled exactly once, last to first)
         }
-        front--;
-        const bool z = a * q == 0;
-        ga.shift_in(sa, a, q, z);
-        gq.shift_in(sq, a, q, z);
-        raw_a = (raw_a >> 3) | (a << (3 * kHist));
-        raw_q = (raw_q >> 7) | ((unsigned long long)q << (7 * kHist));
+        shift_in(a, q);
     };
 #pragma unroll 1
-    for (int t = 0; t < kHist; t++) pull();  // entry k = symbol at p1 - k
+    for (int t = 0; t < kHist; t++) pull((int32_t)p1 - 1 - t);  // entry k = symbol at p1 - k
     ga.init_state(sa);
     gq.init_state(sq);
     const uint32_t pbmax = sa.pb > sq.pb ? sa.pb : sq.pb;
@@ -517,41 +545,94 @@ __device__ __forceinline__ void encode_read_body(const ModelDev& ma, const Model
     const bool direct_a = false;
 #endif
     const uint2* __restrict__ enc_a = direct_a ? ma.aenc : ma.enc;
-    // generator stage: moves the generators to position j (entry 0 = symbol j) and looks the two rows up
-    int32_t j = (int32_t)p1;  // position the generators stand at
-    auto rows_next = [&](uint32_t& row_a, uint32_t& row_q) {
-        j--;
+    uint32_t row_a, row_q;
+    // generator stage, once position j - kHist is in the windows: moves the generators to position j (entry 0 = symbol j)
+    // and looks the two rows up
+    auto gen_step = [&]() {
+        ga.step_back(sa);
+        gq.step_back(sq);
+        pb.retreat();
+        row_a = direct_a ? ga.index(sa, pb.pos, psa) : gen_row<P::kStatic>(ma, sa, ga, pb.pos, psa);
+        row_q = gen_row<P::kStatic>(mq, sq, gq, pb.pos, psq);
+    };
+    auto rows_next = [&](int32_t j) {  // j = p1-1, p1-2, ... in turn (reads are shorter than 2^31)
         row_a = row_q = 0;
         if (j >= (int32_t)p0) {
-            pull();
-            ga.step_back(sa);
-            gq.step_back(sq);
-            pb.retreat();
-            row_a = direct_a ? ga.index(sa, pb.pos, psa) : gen_row<P::kStatic>(ma, sa, ga, pb.pos, psa);
-            row_q = gen_row<P::kStatic>(mq, sq, gq, pb.pos, psq);
+            pull(j - kHist);
+            gen_step();
         }
     };
-    // prologue: rows of position p1-1, its entries, rows of position p1-2
-    uint32_t row_a, row_q;
-    rows_next(row_a, row_q);  // generators at p1-1, entry 0 = symbol p1-1
+    // entries of the position the generators stand at
+    auto entries = [&](uint2& ea_, uint2& eq_) {
+        ea_ = ldg_stream8(enc_a + (row_a * kAcidSyms + (raw_a & 7u)));
+        eq_ = __ldg(mq.enc + (row_q * kQSyms + ((uint32_t)raw_q & 127u)));
+    };
     uint2 ea = make_uint2(0, 0), eq = make_uint2(0, 0);
-    if (p1 > p0) {
-        ea = ldg_stream8(enc_a + (row_a * kAcidSyms + (raw_a & 7u)));
-        eq = __ldg(mq.enc + (row_q * kQSyms + ((uint32_t)raw_q & 127u)));
-    }
-    rows_next(row_a, row_q);  // generators at p1-2
-#pragma unroll 1
-    for (uint32_t i = p1; i-- > p0;) {
-        // entries of position i-1 (generators stand at i-1: entry 0), gathered while position i is coded
-        uint2 ea_n = make_uint2(0, 0), eq_n = make_uint2(0, 0);
-        if (i > p0) {
-            ea_n = ldg_stream8(enc_a + (row_a * kAcidSyms + (raw_a & 7u)));
-            eq_n = __ldg(mq.enc + (row_q * kQSyms + ((uint32_t)raw_q & 127u)));
-        }
-        rows_next(row_a, row_q);  // generators to i-2
+    auto put = [&]() {
         rans_put_bf(S.x0, ea, S.out);  // put_at(0, acid) then put_at(1, q)   compressor.rs:95-96
         rans_put_bf(S.x1, eq, S.out);
         S.out.drain();
+    };
+    // prologue: rows of position p1-1, its entries, rows of position p1-2
+    rows_next((int32_t)p1 - 1);  // generators at p1-1, entry 0 = symbol p1-1
+    if (p1 > p0) entries(ea, eq);
+    rows_next((int32_t)p1 - 2);  // generators at p1-2
+#ifndef IDN_NO_SYM16
+    // Coding position i gathers the entries of i-1 when i > p0, moves the generators to i-2 when i-2 >= p0 and pulls
+    // position i-2-kHist when it is >= 0.  While i >= wlim (i = the last position coded), the next four positions
+    // i-1 .. i-4 do all three, and once the reader stands at a word boundary the four symbols they pull are one word of
+    // each array: that interior runs one word per iteration without the per-position tests; the head (down to the first
+    // word boundary) and the tail run position by position.  The interior also stays above the chunk that holds the
+    // first byte of an array that is not 16-byte aligned (so its loads need no bounds test): its pulls must not reach
+    // below position `skip` of the read.
+    const long long skip = (long long)((0 - reinterpret_cast<uintptr_t>(acids)) & 15) - off;
+    uint32_t wlim = p0 > kHist ? p0 : kHist;
+    if (skip > 0 && (uint32_t)skip + kHist > wlim) wlim = (uint32_t)skip + kHist;
+    wlim += 4 + 2;  // the lowest pull of a word step: (i - 4) - 2 - kHist
+#endif
+    uint32_t i = p1;
+#pragma unroll 1
+    while (i > p0) {
+#ifndef IDN_NO_SYM16
+        // (one word per pass of the outer loop, not a loop of its own: the threads of a warp reach their first word
+        // boundary up to three positions apart, and an inner loop would run their interiors one after the other)
+        if (rs.vec && (rs.left & 3) == 0 && i >= wlim) {
+            rs.peek_word();
+            // some acid > 4 or quality score > 93: flag the read and zero those bytes, as pull() does
+            if ((((rs.ca & 0x7f7f7f7fu) + 0x7b7b7b7bu) | rs.ca | ((rs.cq & 0x7f7f7f7fu) + 0x22222222u) | rs.cq) & 0x80808080u) {
+                S.bad = true;
+                uint32_t ca = 0, cq = 0;
+#pragma unroll 1
+                for (int k = 0; k < 32; k += 8) {
+                    const uint32_t a = (rs.ca >> k) & 0xffu, q = (rs.cq >> k) & 0xffu;
+                    ca |= (a > 4 ? 0u : a) << k;
+                    cq |= (q > 93 ? 0u : q) << k;
+                }
+                rs.ca = ca;
+                rs.cq = cq;
+            }
+            if (C.tinv) C.add_word(rs.ca, rs.cq);
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                uint2 ea_n, eq_n;
+                entries(ea_n, eq_n);  // of position i-2-k
+                shift_in(__byte_perm(rs.ca, 0, 0x4443 - k), __byte_perm(rs.cq, 0, 0x4443 - k));
+                gen_step();  // generators to i-3-k
+                put();       // position i-1-k
+                ea = ea_n;
+                eq = eq_n;
+            }
+            rs.skip_word();
+            i -= 4;
+            continue;
+        }
+#endif
+        i--;
+        // entries of position i-1 (generators stand at i-1: entry 0), gathered while position i is coded
+        uint2 ea_n = make_uint2(0, 0), eq_n = make_uint2(0, 0);
+        if (i > p0) entries(ea_n, eq_n);
+        rows_next((int32_t)i - 2);  // generators to i-2
+        put();
         ea = ea_n;
         eq = eq_n;
     }
@@ -580,12 +661,12 @@ __device__ __forceinline__ void encode_one(const EncodeArgs& A, const ModelDev& 
     const uint32_t len = (uint32_t)(A.read_off[r + 1] - A.read_off[r]);
     EncStream S;
     S.begin(A.scratch + 4ull * A.read_off[r + 1] + kSlotExtra * (r + 1));
-    EncCrc C{A.crc_back ? s_back : nullptr, s_back + 256, 0u, 0u};
+    EncCrc C{A.crc_back ? s_back : nullptr, 0u, 0u};
     encode_read_body<P>(ma, mq, A.acids, A.quals, A.n_symbols, off, len, 0, len, S, C);
     if (A.crc_back) {  // crc(acids | quals) of the read, as crc_read_kernel computes it
         uint32_t x1, x2;  // x^(8 len), x^(16 len) mod P
         if (len < kCrcLenTab) {
-            const uint2 x = __ldg(reinterpret_cast<const uint2*>(A.crc_back + 512) + len);
+            const uint2 x = __ldg(reinterpret_cast<const uint2*>(A.crc_back + 256) + len);
             x1 = x.x;
             x2 = x.y;
         } else {
@@ -621,9 +702,9 @@ __device__ __forceinline__ void encode_one(const EncodeArgs& A, const ModelDev& 
 template <bool kUniform, class P>
 __global__ void __launch_bounds__(128, kUniform ? IDN_ENC_MINB : 1)
 encode_kernel(EncodeArgs A, const ModelDev MA, const ModelDev MQ) {
-    __shared__ uint32_t s_back[512];
+    __shared__ uint32_t s_back[256];
     if (A.crc_back) {
-        for (int i = threadIdx.x; i < 512; i += blockDim.x) s_back[i] = A.crc_back[i];
+        for (int i = threadIdx.x; i < 256; i += blockDim.x) s_back[i] = A.crc_back[i];
         __syncthreads();
     }
     uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -637,9 +718,9 @@ encode_kernel(EncodeArgs A, const ModelDev MA, const ModelDev MQ) {
 template <class P>
 __global__ void __launch_bounds__(128, IDN_ENC_MINB)
 encode_list_kernel(EncodeArgs A, const ModelDev MA, const ModelDev MQ, ReadList L) {
-    __shared__ uint32_t s_back[512];
+    __shared__ uint32_t s_back[256];
     if (A.crc_back) {
-        for (int i = threadIdx.x; i < 512; i += blockDim.x) s_back[i] = A.crc_back[i];
+        for (int i = threadIdx.x; i < 256; i += blockDim.x) s_back[i] = A.crc_back[i];
         __syncthreads();
     }
     const uint32_t n = *L.count;

@@ -159,7 +159,7 @@ __device__ __forceinline__ void encode_lane_one(const EncodeLaneArgs& A, const M
     const ModelDev& ma = kUniform ? MA : A.models[ia];
     const ModelDev& mq = kUniform ? MQ : A.models[iq];
     EncStream S;
-    EncCrc C{nullptr, nullptr, 0u, 0u};  // (the native path takes its CRC partials from crc_read_kernel)
+    EncCrc C{nullptr, 0u, 0u};  // (the native path takes its CRC partials from crc_read_kernel)
     S.begin(A.scratch + 4ull * A.lane_sym[l + 1] + kLaneSlotExtra * ((unsigned long long)l + 1));
     if (A.lane_sym[l + 1] > A.lane_sym[l]) {
         // the last read with a symbol in the lane, then down to the first
