@@ -33,7 +33,8 @@ EXPORTS = [
     "idn_gpu_synth_reads_dev", "idn_gpu_profile", "idn_gpu_profile_read", "idn_gpu_set_lane_symbols", "idn_gpu_set_walk",
     "idn_gpu_fastq_parse", "idn_gpu_fastq_parse_dev", "idn_gpu_fastq_fetch", "idn_gpu_fastq_batch_dev", "idn_gpu_fastq_format",
     "idn_gpu_fastq_format_dev", "idn_gpu_fastq_parse_chunk", "idn_gpu_fastq_chunk_fetch", "idn_gpu_compress_parsed",
-    "idn_gpu_decompress_to_fastq",
+    "idn_gpu_decompress_to_fastq", "idn_gpu_compress_parsed_ids", "idn_gpu_deflate_names", "idn_gpu_deflate_names_dev",
+    "idn_gpu_deflate_names_bound",
 ]
 
 
@@ -161,6 +162,14 @@ def load():
     L.idn_gpu_decompress_to_fastq.argtypes = [vp, vp, vp, vp, vp, u32, i32, vp, u32, vp, vp, u64, u64, i32, vp, u64, C.POINTER(u64),
                                              C.POINTER(u64), C.POINTER(i32)]
     L.idn_gpu_decompress_to_fastq.restype = i32
+    L.idn_gpu_compress_parsed_ids.argtypes = [vp, i32, vp, u32, i32, vp, u64, vp, vp, C.POINTER(CompressStats)]
+    L.idn_gpu_compress_parsed_ids.restype = i32
+    L.idn_gpu_deflate_names.argtypes = [vp, vp, vp, vp, u32, vp, u64, vp]
+    L.idn_gpu_deflate_names.restype = i32
+    L.idn_gpu_deflate_names_dev.argtypes = [vp, vp, vp, vp, u32, vp, u64, vp, vp]
+    L.idn_gpu_deflate_names_dev.restype = i32
+    L.idn_gpu_deflate_names_bound.argtypes = [u64, u64, u32]
+    L.idn_gpu_deflate_names_bound.restype = u64
     L.idn_gpu_set_lane_symbols.argtypes = [vp, u32]
     L.idn_gpu_set_lane_symbols.restype = i32
     L.idn_gpu_set_walk.argtypes = [vp, i32]
@@ -291,6 +300,26 @@ class Context:
         sizes = np.zeros((b.n_reads, len(m)), dtype=np.uint32)
         self.check(self.L.idn_gpu_score(self.h, C.byref(b), _p(m), len(m), _p(sizes)))
         return sizes
+
+    def deflate_names(self, name_off, names, block_first_read, *, out_cap=None):
+        """identifiers slices (0x00 | u32be n | 0x01 | raw Deflate of the block's names joined by '\\n') of every block,
+        Deflated on the device -> (slices, slice_off[n_blocks + 1])"""
+        no = _c(name_off, np.uint64)
+        nm = _c(names, np.uint8)
+        if nm.size == 0:
+            nm = np.zeros(1, dtype=np.uint8)
+        bf = _c(block_first_read, np.uint32)
+        nb = len(bf) - 1
+        if out_cap is None:
+            out_cap = int(self.L.idn_gpu_deflate_names_bound(int(no[-1] - no[0]), len(no) - 1, nb))
+        out = np.zeros(max(out_cap, 1), dtype=np.uint8)
+        so = np.zeros(nb + 1, dtype=np.uint64)
+        rc = self.L.idn_gpu_deflate_names(self.h, nm.ctypes.data, no.ctypes.data, bf.ctypes.data, nb, out.ctypes.data, out_cap, so.ctypes.data)
+        if rc != OK:
+            e = IdnGpuError(rc, self.L.idn_gpu_last_error(self.h).decode())
+            e.required = int(so[-1])
+            raise e
+        return out[:int(so[-1])], so
 
     def compress_blocks(self, read_off, acids, quals, block_first_read, models, *, fast=False, prefix_len=None,
                         name_off=None, names=None, out_cap=None, mode=MODE_COMPAT):

@@ -156,6 +156,7 @@ extern "C" void idn_host_params_default(idn_host_params* p) {
     p->text_chunk_bytes = d.text_chunk_bytes;
     p->n_devices = 0;
     for (int32_t& v : p->devices) v = 0;
+    p->identifiers_on_device = d.identifiers_on_device;
 }
 
 extern "C" int32_t idn_host_compressor_new(const idn_host_model* const* models, uint32_t n_models, const idn_host_params* params,
@@ -177,6 +178,7 @@ extern "C" int32_t idn_host_compressor_new(const idn_host_model* const* models, 
                                     .batch_blocks(params->batch_blocks)
                                     .lane_symbols(params->lane_symbols)
                                     .text_chunk_bytes(params->text_chunk_bytes ? params->text_chunk_bytes : (256ull << 20))
+                                    .identifiers_on_device(params->identifiers_on_device != 0)
                                     .build();
         auto h = std::make_unique<idn_host_compressor>();
         idn_host_compressor* raw = h.get();

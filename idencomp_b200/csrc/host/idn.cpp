@@ -350,6 +350,8 @@ IdnCompressorParamsBuilder& IdnCompressorParamsBuilder::quality(uint8_t v) {
 IdnCompressor::IdnCompressor(Sink sink, IdnCompressorParams params) : sink_(std::move(sink)), params_(std::move(params)) {
     if (params_.fast) params_.quality = 1;  // IdnCompressorParamsBuilder::fast (idn/compressor.rs:244-251)
     if (params_.mode != IDN_MODE_COMPAT && params_.mode != IDN_MODE_NATIVE) throw IdnError(IDN_E_INVALID_STATE, "unknown container mode");
+    if (params_.identifiers_on_device && params_.include_identifiers && params_.quality >= 8)
+        throw IdnError(IDN_E_UNSUPPORTED, "identifiers_on_device: quality 8-9 codes identifiers with Brotli, which has no device codec");
     if (params_.devices.empty()) params_.devices.assign(1, 0);
     if (params_.batch_blocks == 0) params_.batch_blocks = 1;
     for (int32_t d : params_.devices) {
@@ -544,8 +546,20 @@ IdnCompressor::Result IdnCompressor::compress_batch(Worker& w, const Batch& bt) 
     const uint64_t n_reads = bt.block_first.back();
     std::vector<std::vector<uint8_t>> name_slices(n_blocks);
     std::vector<uint32_t> prefix(n_blocks, 0);
-    if (params_.include_identifiers)
+    std::shared_ptr<PinnedBuf> dev_slices;  // identifiers_on_device: the slices back to back ...
+    std::vector<uint64_t> slice_off;        // ... block k's at slice_off[k]
+    if (params_.include_identifiers && params_.identifiers_on_device) {
+        Span sp(T_NDEFLATE);
+        const uint8_t* names = bt.names.empty() ? reinterpret_cast<const uint8_t*>("") : bt.names.data();
+        const uint64_t cap = idn_gpu_deflate_names_bound(bt.name_off[n_reads] - bt.name_off[0], n_reads, n_blocks);
+        dev_slices = pool_.get(cap);
+        slice_off.resize(n_blocks + 1);
+        int32_t rc = idn_gpu_deflate_names(w.dev.ctx(), names, bt.name_off.data(), bt.block_first.data(), n_blocks, dev_slices->p, cap, slice_off.data());
+        if (rc) w.dev.raise(rc);
+        for (uint32_t k = 0; k < n_blocks; k++) prefix[k] = (uint32_t)(slice_off[k + 1] - slice_off[k]);
+    } else if (params_.include_identifiers) {
         identifier_slices(params_.quality, params_.thread_num, n_blocks, bt.block_first.data(), bt.names.data(), bt.name_off.data(), name_slices, prefix);
+    }
     res.prefix_total = std::accumulate(prefix.begin(), prefix.end(), (uint64_t)0);
     idn_batch b{};
     b.n_reads = n_reads;
@@ -579,7 +593,7 @@ IdnCompressor::Result IdnCompressor::compress_batch(Worker& w, const Batch& bt) 
         break;
     }
     for (uint32_t k = 0; k < n_blocks; k++)
-        if (prefix[k]) std::memcpy(res.buf->p + block_off[k] + 8, name_slices[k].data(), prefix[k]);
+        if (prefix[k]) std::memcpy(res.buf->p + block_off[k] + 8, dev_slices ? dev_slices->p + slice_off[k] : name_slices[k].data(), prefix[k]);
     res.out_bytes = st.out_bytes;
     res.payload_bytes = st.payload_bytes;
     res.acid_switches = st.acid_switches;
@@ -808,6 +822,7 @@ IdnCompressor::Result IdnCompressor::compress_parsed(Worker& w, uint32_t n_block
                                                      uint64_t n_name_bytes) const {
     WorkerLease<Worker> lease(w, true);
     Result res;
+    if (params_.include_identifiers && params_.identifiers_on_device) return compress_parsed_ids(w, n_blocks, n_reads, n_symbols, n_name_bytes);
     std::vector<std::vector<uint8_t>> name_slices(n_blocks);
     std::vector<uint32_t> prefix(n_blocks, 0);
     if (params_.include_identifiers) {
@@ -843,6 +858,40 @@ IdnCompressor::Result IdnCompressor::compress_parsed(Worker& w, uint32_t n_block
     }
     for (uint32_t k = 0; k < n_blocks; k++)
         if (prefix[k]) std::memcpy(res.buf->p + block_off[k] + 8, name_slices[k].data(), prefix[k]);
+    res.out_bytes = st.out_bytes;
+    res.payload_bytes = st.payload_bytes;
+    res.acid_switches = st.acid_switches;
+    res.q_switches = st.q_switches;
+    res.blocks = n_blocks;
+    return res;
+}
+
+// compress_parsed with identifiers_on_device: the library Deflates the names where the parse left them and puts the slices
+// into the container; the slice lengths are read back from their headers for the statistics
+IdnCompressor::Result IdnCompressor::compress_parsed_ids(Worker& w, uint32_t n_blocks, uint64_t n_reads, uint64_t n_symbols,
+                                                         uint64_t n_name_bytes) const {
+    Result res;
+    const uint64_t ids_bound = idn_gpu_deflate_names_bound(n_name_bytes, n_reads, n_blocks);
+    const uint64_t bound = idn_gpu_compress_bound(n_reads, n_symbols, n_blocks, ids_bound);
+    uint64_t cap = std::min<uint64_t>(bound, n_symbols + n_symbols / 4 + 24 * n_reads + 64ull * n_blocks + n_name_bytes / 2 + 4096);
+    std::vector<uint64_t> block_off(n_blocks + 1);
+    idn_compress_stats st{};
+    Span sp_c(T_CPARSED);
+    for (;;) {
+        res.buf = pool_.get(cap);
+        int32_t rc = idn_gpu_compress_parsed_ids(w.dev.ctx(), params_.mode, w.dev.handles().data(), (uint32_t)w.dev.handles().size(),
+                                                 params_.fast ? 1 : 0, res.buf->p, cap, block_off.data(), nullptr, &st);
+        if (rc == IDN_E_NOSPACE && cap < bound) {
+            cap = bound;
+            continue;
+        }
+        if (rc) w.dev.raise(rc);
+        break;
+    }
+    for (uint32_t k = 0; k < n_blocks; k++) {  // 0x00 | u32be n | 0x01 | n bytes
+        const uint8_t* h = res.buf->p + block_off[k] + 9;
+        res.prefix_total += 6 + ((uint64_t)h[0] << 24 | (uint64_t)h[1] << 16 | (uint64_t)h[2] << 8 | h[3]);
+    }
     res.out_bytes = st.out_bytes;
     res.payload_bytes = st.payload_bytes;
     res.acid_switches = st.acid_switches;

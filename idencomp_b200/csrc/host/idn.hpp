@@ -65,6 +65,9 @@ struct IdnCompressorParams {
     uint32_t batch_blocks = 32;      // blocks per device call
     uint32_t lane_symbols = 2048;    // native mode lane quantum
     uint64_t text_chunk_bytes = 256ull << 20;  // add_fastq_text: bytes of FASTQ text per device call
+    // identifiers slices Deflated on the device (idn_gpu_deflate_names) instead of by the host's zlib: other Deflate bytes,
+    // somewhat larger, the same names after inflation.  Not available for the Brotli slices of quality 8-9.
+    bool identifiers_on_device = false;
 };
 
 class IdnCompressorParamsBuilder {
@@ -81,6 +84,7 @@ public:
     IdnCompressorParamsBuilder& batch_blocks(uint32_t v) { p_.batch_blocks = v ? v : 1; return *this; }
     IdnCompressorParamsBuilder& lane_symbols(uint32_t v) { p_.lane_symbols = v; return *this; }
     IdnCompressorParamsBuilder& text_chunk_bytes(uint64_t v) { p_.text_chunk_bytes = v ? v : 1; return *this; }
+    IdnCompressorParamsBuilder& identifiers_on_device(bool v) { p_.identifiers_on_device = v; return *this; }
     IdnCompressorParams build() const { return p_; }
 
 private:
@@ -198,6 +202,7 @@ private:
     };
     size_t consume_text(const uint8_t* buf, size_t total, bool final);
     Result compress_parsed(Worker& w, uint32_t n_blocks, uint64_t n_reads, uint64_t n_symbols, uint64_t n_name_bytes) const;
+    Result compress_parsed_ids(Worker& w, uint32_t n_blocks, uint64_t n_reads, uint64_t n_symbols, uint64_t n_name_bytes) const;
     void make_block();
     void flush_batch();  // hands the batch under construction to the next device
     void commit(bool all);  // writes finished batches in order (the reference's IdnBlockLock, idn/common.rs:10-57)

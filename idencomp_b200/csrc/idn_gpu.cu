@@ -14,6 +14,7 @@
 
 #include "idn_fastq.cuh"
 #include "idn_native.cuh"
+#include "idn_deflate.cuh"
 
 using namespace idn;
 
@@ -138,6 +139,8 @@ struct idn_gpu_ctx {
     DevBuf s_acids, s_quals, s_readoff, s_blockfirst, s_prefix, s_names, s_nameoff, s_out, s_blockoff, s_crc, s_stats,
         s_sizes, s_blocks, s_blocklen, s_aout, s_qout, s_offout, s_status, s_idx;
     DevBuf w_bucket, w_list;       // per-read selection: reads bucketed by model pair (cnt | base | cursor, read list)
+    // identifiers Deflate (idn_deflate.cuh): per-block tables, joined names, candidates, tokens, segment records, slices
+    DevBuf z_blk, z_joined, z_cand, z_tok, z_ntok, z_rec, z_segblock, z_segoff, z_out;
     bool bucket_pairs = true;      // IDN_NO_BUCKETS=1: the run-time generic kernels over all reads instead (for comparison)
     uint64_t resident_bytes = 0;   // container bytes idn_gpu_index_blocks / the decoder left in s_blocks ...
     uint32_t resident_blocks = 0;  // ... and how many blocks they are (0: nothing a decode call may reuse)
@@ -459,7 +462,9 @@ extern "C" void idn_gpu_destroy(idn_gpu_ctx* ctx) {
                       &ctx->f_blockfirst, &ctx->f_nxt, &ctx->w_bucket, &ctx->w_list,
                       &ctx->s_acids,   &ctx->s_quals,   &ctx->s_readoff, &ctx->s_blockfirst, &ctx->s_prefix, &ctx->s_names,
                       &ctx->s_nameoff, &ctx->s_out,     &ctx->s_blockoff, &ctx->s_crc,       &ctx->s_stats,  &ctx->s_sizes,
-                      &ctx->s_blocks,  &ctx->s_blocklen, &ctx->s_aout,    &ctx->s_qout,    &ctx->s_offout,     &ctx->s_status, &ctx->s_idx};
+                      &ctx->s_blocks,  &ctx->s_blocklen, &ctx->s_aout,    &ctx->s_qout,    &ctx->s_offout,     &ctx->s_status, &ctx->s_idx,
+                      &ctx->z_blk, &ctx->z_joined, &ctx->z_cand, &ctx->z_tok, &ctx->z_ntok, &ctx->z_rec, &ctx->z_segblock,
+                      &ctx->z_segoff, &ctx->z_out};
     for (DevBuf* b : bufs) b->release();
     pipe_destroy(ctx->pipe);
     cudaFree(ctx->d_models);

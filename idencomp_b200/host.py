@@ -36,7 +36,7 @@ class Params(C.Structure):
     _fields_ = [("max_block_total_len", C.c_uint32), ("thread_num", C.c_uint32), ("include_identifiers", C.c_int32),
                 ("quality", C.c_uint32), ("fast", C.c_int32), ("device", C.c_int32), ("mode", C.c_int32),
                 ("batch_blocks", C.c_uint32), ("lane_symbols", C.c_uint32), ("text_chunk_bytes", C.c_uint64), ("n_devices", C.c_uint32),
-                ("devices", C.c_int32 * 16)]
+                ("devices", C.c_int32 * 16), ("identifiers_on_device", C.c_int32)]
 
 _LIB = None
 
@@ -225,11 +225,13 @@ class IdnCompressor:
     """idencomp::IdnCompressor (idn/compressor.rs:443-585) writing to memory.
 
         c = IdnCompressor(models, quality=7, include_identifiers=True)   # IdnCompressor::with_params
+        identifiers_on_device=True: the identifiers slices are Deflated on the GPU instead of by the host's zlib
         c.add_sequence(b"name", acids, quals) ; ... ; idn = c.finish()
     """
 
     def __init__(self, models, *, max_block_total_len=4 * 1024 * 1024, thread_num=0, include_identifiers=True, quality=7,
-                 fast=False, device=0, devices=None, mode=capi.MODE_COMPAT, batch_blocks=32, lane_symbols=2048, text_chunk_bytes=0):
+                 fast=False, device=0, devices=None, mode=capi.MODE_COMPAT, batch_blocks=32, lane_symbols=2048, text_chunk_bytes=0,
+                 identifiers_on_device=False):
         self.L = load()
         p = Params()
         self.L.idn_host_params_default(C.byref(p))
@@ -237,6 +239,7 @@ class IdnCompressor:
         p.quality, p.fast, p.device, p.mode, p.batch_blocks, p.lane_symbols = quality, int(fast), device, mode, batch_blocks, lane_symbols
         if text_chunk_bytes:
             p.text_chunk_bytes = text_chunk_bytes
+        p.identifiers_on_device = int(identifiers_on_device)
         if devices:  # several GPUs share the file: same container, whatever their number
             p.n_devices = len(devices)
             for i, d in enumerate(devices):

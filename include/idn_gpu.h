@@ -284,6 +284,11 @@ int32_t idn_gpu_fastq_chunk_fetch(idn_gpu_ctx *ctx, uint8_t *names, uint64_t *na
 int32_t idn_gpu_compress_parsed(idn_gpu_ctx *ctx, int32_t mode, const idn_model_t *models, uint32_t n_models, int32_t fast,
                                 int32_t with_names, const uint32_t *prefix_len, uint8_t *out, uint64_t out_cap,
                                 uint64_t *block_off, uint32_t *block_crc, idn_compress_stats *stats);
+/* idn_gpu_compress_parsed with the identifiers Deflated on the device (idn_gpu_deflate_names_dev) and put into the room after
+ * each block header there: `out` comes back complete, the names never leave the device, the block CRCs cover them. */
+int32_t idn_gpu_compress_parsed_ids(idn_gpu_ctx *ctx, int32_t mode, const idn_model_t *models, uint32_t n_models, int32_t fast,
+                                    uint8_t *out, uint64_t out_cap, uint64_t *block_off, uint32_t *block_crc,
+                                    idn_compress_stats *stats);
 /* idn_gpu_decompress_blocks + FastqWriter: the FASTQ text of the decoded reads into `text` (the symbols stay on the
  * device); names / name_off = the identifiers the caller inflated (optional) */
 int32_t idn_gpu_decompress_to_fastq(idn_gpu_ctx *ctx, const uint8_t *blocks, const uint64_t *block_off,
@@ -292,6 +297,24 @@ int32_t idn_gpu_decompress_to_fastq(idn_gpu_ctx *ctx, const uint8_t *blocks, con
                                     const uint64_t *name_off, uint64_t reads_cap, uint64_t symbols_cap,
                                     int32_t title_with_separator, uint8_t *text, uint64_t text_cap, uint64_t *text_len,
                                     uint64_t *n_reads_out, int32_t *bad_block);
+
+/* ---- identifiers slices: raw Deflate (RFC 1951) on the device ----------------------------------------------------------
+ * For each block b (reads [block_first_read[b], block_first_read[b+1]), block_first_read[0] = 0, names[name_off[r] ..
+ * name_off[r+1]) per read) the bytes write_identifiers emits (compressor_block.rs:146-206) with Deflate:
+ *     0x00 | u32be n | 0x01 | n bytes of raw Deflate of the block's names joined by '\n'
+ * at out[slice_off[b] .. slice_off[b+1]).  The Deflate bytes are not zlib's: the names are coded in segments of 64 KiB,
+ * each one block with its own Huffman code, the segments of a block joined by empty stored blocks; any inflater reads
+ * them.  They depend only on the block's names (not on the other blocks of the call, the device or scheduling).
+ * IDN_E_INVALID_ARG for a name_off or block_first_read that is not monotone or a block_first_read[0] != 0;
+ * IDN_E_NOSPACE when out_cap is too small, slice_off[n_blocks] then holds the size needed.  The _dev form takes DEVICE
+ * pointers and synchronises `stream` three times to size its work; the other stages them and returns when done. */
+int32_t idn_gpu_deflate_names(idn_gpu_ctx *ctx, const uint8_t *names, const uint64_t *name_off, const uint32_t *block_first_read,
+                              uint32_t n_blocks, uint8_t *out, uint64_t out_cap, uint64_t *slice_off /*[n_blocks+1]*/);
+int32_t idn_gpu_deflate_names_dev(idn_gpu_ctx *ctx, const uint8_t *names, const uint64_t *name_off, const uint32_t *block_first_read,
+                                  uint32_t n_blocks, uint8_t *out, uint64_t out_cap, uint64_t *slice_off /*[n_blocks+1]*/,
+                                  void *stream);
+/* upper bound of slice_off[n_blocks] for any names of this shape (name_bytes = name_off[R] - name_off[0]) */
+uint64_t idn_gpu_deflate_names_bound(uint64_t name_bytes, uint64_t n_reads, uint32_t n_blocks);
 
 /* ---- per-kernel timing (CUDA events on the launching stream; what bench.py's roofline line is made of) ----
  * idn_gpu_profile(ctx, 1) starts recording an event after every kernel launch of the *_dev entry points;

@@ -65,6 +65,8 @@ typedef struct {                    /* IdnCompressorParamsBuilder, idn/compresso
     uint32_t n_devices;             /* > 0: the GPUs that share the file (batches go round robin, results are committed in block
                                        order; the container does not depend on the device count) */
     int32_t devices[16];
+    int32_t identifiers_on_device;  /* default 0; != 0: identifiers slices Deflated on the device (idn_gpu_deflate_names),
+                                       IDN_E_UNSUPPORTED with include_identifiers at quality 8-9 (Brotli) */
 } idn_host_params;
 void idn_host_params_default(idn_host_params *p);
 /* IdnCompressor::with_params over an in-memory writer; `models` is the ModelProvider (order = provider order) */
