@@ -34,7 +34,8 @@ EXPORTS = [
     "idn_gpu_fastq_parse", "idn_gpu_fastq_parse_dev", "idn_gpu_fastq_fetch", "idn_gpu_fastq_batch_dev", "idn_gpu_fastq_format",
     "idn_gpu_fastq_format_dev", "idn_gpu_fastq_parse_chunk", "idn_gpu_fastq_chunk_fetch", "idn_gpu_compress_parsed",
     "idn_gpu_decompress_to_fastq", "idn_gpu_compress_parsed_ids", "idn_gpu_deflate_names", "idn_gpu_deflate_names_dev",
-    "idn_gpu_deflate_names_bound",
+    "idn_gpu_deflate_names_bound", "idn_gpu_inflate_names", "idn_gpu_inflate_names_fetch", "idn_gpu_set_inflate_range",
+    "idn_gpu_decompress_blocks_ids", "idn_gpu_decompress_to_fastq_ids",
 ]
 
 
@@ -70,6 +71,13 @@ class FastqInfo(C.Structure):
 class FastqChunk(C.Structure):
     _fields_ = [("n_reads", C.c_uint64), ("n_symbols", C.c_uint64), ("n_name_bytes", C.c_uint64), ("n_blocks", C.c_uint32),
                 ("error_kind", C.c_int32), ("bad_record", C.c_uint64), ("consumed_text", C.c_uint64)]
+
+
+class InflateStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("n_streams", "n_chunks", "n_speculative", "n_joined", "serial_bytes", "in_bytes")]
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
 
 
 FASTQ_ERRORS = {1: "InvalidFormat", 2: "InvalidAcid", 3: "InvalidQualityScore", 4: "AcidAndQualityScoreLengthMismatch",
@@ -170,6 +178,17 @@ def load():
     L.idn_gpu_deflate_names_dev.restype = i32
     L.idn_gpu_deflate_names_bound.argtypes = [u64, u64, u32]
     L.idn_gpu_deflate_names_bound.restype = u64
+    L.idn_gpu_inflate_names.argtypes = [vp, vp, vp, vp, u32, vp, u64, C.POINTER(u64), C.POINTER(i32), C.POINTER(InflateStats)]
+    L.idn_gpu_inflate_names.restype = i32
+    L.idn_gpu_inflate_names_fetch.argtypes = [vp, vp, vp]
+    L.idn_gpu_inflate_names_fetch.restype = i32
+    L.idn_gpu_set_inflate_range.argtypes = [vp, u32]
+    L.idn_gpu_set_inflate_range.restype = i32
+    L.idn_gpu_decompress_blocks_ids.argtypes = [vp, vp, vp, vp, vp, u32, i32, vp, u32, vp, vp, vp, u64, u64, C.POINTER(i32)]
+    L.idn_gpu_decompress_blocks_ids.restype = i32
+    L.idn_gpu_decompress_to_fastq_ids.argtypes = [vp, vp, vp, vp, vp, u32, i32, vp, u32, u64, u64, i32, vp, u64, C.POINTER(u64),
+                                                  C.POINTER(u64), C.POINTER(i32)]
+    L.idn_gpu_decompress_to_fastq_ids.restype = i32
     L.idn_gpu_set_lane_symbols.argtypes = [vp, u32]
     L.idn_gpu_set_lane_symbols.restype = i32
     L.idn_gpu_set_walk.argtypes = [vp, i32]
@@ -320,6 +339,34 @@ class Context:
             e.required = int(so[-1])
             raise e
         return out[:int(so[-1])], so
+
+    def set_inflate_range(self, n: int):
+        """compressed bytes per range of the parallel inflate (idn_gpu_set_inflate_range)"""
+        self.check(self.L.idn_gpu_set_inflate_range(self.h, n))
+
+    def inflate_names(self, blocks, block_off, block_first_read, *, block_len=None, resident=False):
+        """the blocks' Identifiers slices inflated and split into names on the device -> (names, name_off, stats).
+        blocks: payloads as idn_gpu_decompress_blocks takes them; resident=True passes blocks == NULL (the bytes of the last
+        index_blocks call).  A failure raises IdnGpuError with .bad_block and .stats."""
+        bo = _c(block_off, np.uint64)
+        bl = None if block_len is None else _c(block_len, np.uint32)
+        bf = _c(block_first_read, np.uint32)
+        blk = None if resident else _c(blocks, np.uint8)
+        if blk is not None and blk.size == 0:
+            blk = np.zeros(1, dtype=np.uint8)
+        n_reads = int(bf[-1])
+        nb, bad, st = C.c_uint64(0), C.c_int32(-1), InflateStats()
+        rc = self.L.idn_gpu_inflate_names(self.h, _p(blk), bo.ctypes.data, _p(bl), len(bo) - 1, bf.ctypes.data, n_reads, C.byref(nb),
+                                          C.byref(bad), C.byref(st))
+        if rc != OK:
+            e = IdnGpuError(rc, self.L.idn_gpu_last_error(self.h).decode())
+            e.bad_block = int(bad.value)
+            e.stats = st.as_dict()
+            raise e
+        names = np.zeros(max(1, nb.value), dtype=np.uint8)
+        name_off = np.zeros(n_reads + 1, dtype=np.uint64)
+        self.check(self.L.idn_gpu_inflate_names_fetch(self.h, names.ctypes.data, name_off.ctypes.data))
+        return names[:nb.value], name_off, st.as_dict()
 
     def compress_blocks(self, read_off, acids, quals, block_first_read, models, *, fast=False, prefix_len=None,
                         name_off=None, names=None, out_cap=None, mode=MODE_COMPAT):

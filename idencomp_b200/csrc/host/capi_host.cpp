@@ -228,15 +228,16 @@ extern "C" int32_t idn_host_compressor_add_text(idn_host_compressor* c, const ui
     });
 }
 
-extern "C" int32_t idn_host_decompress_text(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
+extern "C" int32_t idn_host_decompress_text_ex(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
                                             uint32_t thread_num, int32_t title_with_separator, const uint8_t* idn, uint64_t idn_len,
-                                            uint8_t** text, uint64_t* text_len) {
+                                            uint8_t** text, uint64_t* text_len, const idn_host_decompress_params* dparams) {
     if (!text || !text_len || (!idn && idn_len) || (n_models && !models)) return set_err(IDN_E_INVALID_ARG, "NULL argument");
     *text = nullptr;
     *text_len = 0;
     return guarded([&] {
         IdnDecompressorParams p;
         p.model_provider = provider_of(models, n_models);
+        p.identifiers_on_device = dparams && dparams->identifiers_on_device;
         p.thread_num = thread_num;
         if (device >= 0) {
             p.devices.assign(1, device);
@@ -283,14 +284,15 @@ extern "C" void idn_host_release_cached(void) { release_cached_resources(); }
 
 // the same into the caller's buffer (page-locked and touched, if the caller wants the full rate); IDN_E_NOSPACE with
 // *text_len = bytes written so far when it is too small
-extern "C" int32_t idn_host_decompress_text_into(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
+extern "C" int32_t idn_host_decompress_text_into_ex(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
                                                  uint32_t thread_num, int32_t title_with_separator, const uint8_t* idn, uint64_t idn_len,
-                                                 uint8_t* text, uint64_t cap, uint64_t* text_len) {
+                                                 uint8_t* text, uint64_t cap, uint64_t* text_len, const idn_host_decompress_params* dparams) {
     if (!text_len || (!text && cap) || (!idn && idn_len) || (n_models && !models)) return set_err(IDN_E_INVALID_ARG, "NULL argument");
     *text_len = 0;
     return guarded([&] {
         IdnDecompressorParams p;
         p.model_provider = provider_of(models, n_models);
+        p.identifiers_on_device = dparams && dparams->identifiers_on_device;
         p.thread_num = thread_num;
         if (device >= 0) {
             p.devices.assign(1, device);
@@ -325,15 +327,16 @@ struct idn_host_text_reader {
     std::shared_ptr<PinnedBuf> piece;
     bool sep = false;
 };
-extern "C" int32_t idn_host_text_reader_new(const idn_host_model* const* models, uint32_t n_models, const int32_t* devices, uint32_t n_devices,
+extern "C" int32_t idn_host_text_reader_new_ex(const idn_host_model* const* models, uint32_t n_models, const int32_t* devices, uint32_t n_devices,
                                             uint32_t batch_blocks, uint32_t thread_num, int32_t title_with_separator, const uint8_t* idn,
-                                            uint64_t idn_len, idn_host_text_reader** out) {
+                                            uint64_t idn_len, idn_host_text_reader** out, const idn_host_decompress_params* dparams) {
     if (!out || (!idn && idn_len) || (n_models && !models) || (n_devices && !devices)) return set_err(IDN_E_INVALID_ARG, "NULL argument");
     *out = nullptr;
     return guarded([&] {
         auto r = std::make_unique<idn_host_text_reader>();
         IdnDecompressorParams p;
         p.model_provider = provider_of(models, n_models);
+        p.identifiers_on_device = dparams && dparams->identifiers_on_device;
         p.thread_num = thread_num;
         if (n_devices) p.devices.assign(devices, devices + n_devices);
         p.batch_blocks = batch_blocks ? batch_blocks : 32;
@@ -403,13 +406,14 @@ extern "C" void idn_host_compressor_stats(const idn_host_compressor* c, uint64_t
 
 extern "C" void idn_host_compressor_free(idn_host_compressor* c) { delete c; }
 
-extern "C" int32_t idn_host_decompress(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
-                                       const uint8_t* idn, uint64_t idn_len, idn_host_decoded** out) {
+extern "C" int32_t idn_host_decompress_ex(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
+                                       const uint8_t* idn, uint64_t idn_len, idn_host_decoded** out, const idn_host_decompress_params* dparams) {
     if (!out || (!idn && idn_len) || (n_models && !models)) return set_err(IDN_E_INVALID_ARG, "NULL argument");
     *out = nullptr;
     return guarded([&] {
         IdnDecompressorParams p;
         p.model_provider = provider_of(models, n_models);
+        p.identifiers_on_device = dparams && dparams->identifiers_on_device;
         if (device >= 0) {
             p.devices.assign(1, device);
         } else {
@@ -500,4 +504,28 @@ extern "C" uint32_t idn_host_rank(const uint32_t* cost, uint64_t n_values, uint3
     std::vector<size_t> best = rank_models(c, n_values, n_models, model_num);
     for (size_t k = 0; k < best.size(); k++) models_out[k] = (uint32_t)best[k];
     return (uint32_t)best.size();
+}
+
+// the forms without decompressor parameters: the defaults (identifiers inflated on the host)
+extern "C" int32_t idn_host_decompress_text(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
+                                            uint32_t thread_num, int32_t title_with_separator, const uint8_t* idn, uint64_t idn_len,
+                                            uint8_t** text, uint64_t* text_len) {
+    return idn_host_decompress_text_ex(models, n_models, device, batch_blocks, thread_num, title_with_separator, idn, idn_len, text, text_len, nullptr);
+}
+
+extern "C" int32_t idn_host_decompress_text_into(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
+                                                 uint32_t thread_num, int32_t title_with_separator, const uint8_t* idn, uint64_t idn_len,
+                                                 uint8_t* text, uint64_t cap, uint64_t* text_len) {
+    return idn_host_decompress_text_into_ex(models, n_models, device, batch_blocks, thread_num, title_with_separator, idn, idn_len, text, cap, text_len, nullptr);
+}
+
+extern "C" int32_t idn_host_text_reader_new(const idn_host_model* const* models, uint32_t n_models, const int32_t* devices, uint32_t n_devices,
+                                            uint32_t batch_blocks, uint32_t thread_num, int32_t title_with_separator, const uint8_t* idn,
+                                            uint64_t idn_len, idn_host_text_reader** out) {
+    return idn_host_text_reader_new_ex(models, n_models, devices, n_devices, batch_blocks, thread_num, title_with_separator, idn, idn_len, out, nullptr);
+}
+
+extern "C" int32_t idn_host_decompress(const idn_host_model* const* models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
+                                       const uint8_t* idn, uint64_t idn_len, idn_host_decoded** out) {
+    return idn_host_decompress_ex(models, n_models, device, batch_blocks, idn, idn_len, out, nullptr);
 }

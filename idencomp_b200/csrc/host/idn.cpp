@@ -146,10 +146,10 @@ struct Brotli {
 // ---- IDN_HOST_TRACE=1: wall time per stage of the host mirror, summed over threads, printed when an object closes -----------
 namespace {
 struct Trace {
-    static constexpr int kN = 16;
+    static constexpr int kN = 17;
     const char* name[kN] = {"parse_chunk", "first_block_select", "names_fetch", "names_deflate", "compress_parsed", "compress_blocks",
                             "sink", "read_raw", "index_blocks", "names_inflate", "decode", "wait_worker", "open", "initialize", "wait_result",
-                            "close"};
+                            "close", "names_inflate_device"};
     std::atomic<uint64_t> ns[kN];
     std::atomic<uint64_t> calls[kN];
     bool on = std::getenv("IDN_HOST_TRACE") != nullptr;
@@ -178,7 +178,8 @@ struct Span {
     }
 };
 std::atomic<size_t> g_raw_hint{1 << 20};  // bytes of the largest batch of container bytes read so far (sizes the next buffer)
-enum { T_PARSE, T_SELECT, T_NFETCH, T_NDEFLATE, T_CPARSED, T_CBLOCKS, T_SINK, T_READRAW, T_INDEX, T_NINFLATE, T_DECODE, T_WAIT, T_OPEN, T_INIT, T_WAITRES, T_CLOSE };
+enum { T_PARSE, T_SELECT, T_NFETCH, T_NDEFLATE, T_CPARSED, T_CBLOCKS, T_SINK, T_READRAW, T_INDEX, T_NINFLATE, T_DECODE, T_WAIT, T_OPEN, T_INIT, T_WAITRES, T_CLOSE,
+       T_NINFLATE_DEV };
 }  // namespace
 
 // ---- page-locked buffers -------------------------------------------------------------------------------------------------
@@ -1118,6 +1119,31 @@ void IdnDecompressor::inflate_names(const RawBatch& rb, const std::vector<uint64
     });
 }
 
+// identifiers_on_device: the batch's Identifiers slices inflated on the device, from the container bytes idn_gpu_index_blocks
+// left there; the names stay on the device for the _ids decode calls (and come back when `fetch`).  A Brotli slice makes
+// the library decline (IDN_E_UNSUPPORTED): false, and the batch takes the host's inflate_names.
+bool IdnDecompressor::inflate_names_device(Worker& w, const RawBatch& rb, const std::vector<uint64_t>& off,
+                                           const std::vector<uint32_t>& block_first, uint64_t n_reads, DecodedBatch& out, bool fetch,
+                                           uint64_t* n_name_bytes) const {
+    Span sp(T_NINFLATE_DEV);
+    const uint32_t n_blocks = (uint32_t)rb.off.size();
+    uint64_t n_bytes = 0;
+    int32_t bad = -1;
+    idn_inflate_stats st{};
+    int32_t rc = idn_gpu_inflate_names(w.dev.ctx(), nullptr, off.data(), rb.len.data(), n_blocks, block_first.data(), n_reads, &n_bytes, &bad, &st);
+    if (rc == IDN_E_UNSUPPORTED) return false;
+    if (rc) w.dev.raise(rc);
+    out.any_names = st.n_streams > 0;
+    *n_name_bytes = n_bytes;
+    if (fetch) {
+        out.names.resize(n_bytes);
+        out.name_off.assign(n_reads + 1, 0);
+        rc = idn_gpu_inflate_names_fetch(w.dev.ctx(), out.names.data(), out.name_off.data());
+        if (rc) w.dev.raise(rc);
+    }
+    return true;
+}
+
 IdnDecompressor::DecodedBatch IdnDecompressor::decode_batch(Worker& w, const RawBatch& rb) const {
     std::lock_guard<std::mutex> lock(w.mu);
     DecodedBatch out;
@@ -1136,7 +1162,10 @@ IdnDecompressor::DecodedBatch IdnDecompressor::decode_batch(Worker& w, const Raw
                                   block_first.data());
     }
     if (rc) w.dev.raise(rc);
-    {
+    // next_batch / next_sequence hand the names out: the device's come back to the host
+    uint64_t dev_name_bytes = 0;
+    const bool on_dev = params_.identifiers_on_device && inflate_names_device(w, rb, off, block_first, tot.n_reads, out, true, &dev_name_bytes);
+    if (!on_dev) {
         Span sp(T_NINFLATE);
         inflate_names(rb, off, block_first, tot.n_reads, out);
     }
@@ -1146,11 +1175,18 @@ IdnDecompressor::DecodedBatch IdnDecompressor::decode_batch(Worker& w, const Raw
     out.read_off.assign(tot.n_reads + 1, 0);
     int32_t bad = -1;
     if (out.names.empty()) out.names.push_back(0);
-    // with identifiers the call is not pipelined and can use the bytes idn_gpu_index_blocks left on the device (blocks == NULL)
-    rc = idn_gpu_decompress_blocks(w.dev.ctx(), out.any_names ? nullptr : rb.base, off.data(), rb.len.data(), rb.crc.data(), n_blocks, mode, handles.data(),
-                                   (uint32_t)handles.size(), out.any_names ? out.names.data() : nullptr,
-                                   out.any_names ? out.name_off.data() : nullptr, out.acids.data(), out.quals.data(), out.read_off.data(),
-                                   tot.n_reads, tot.n_symbols, &bad);
+    if (on_dev) {
+        // the block CRCs read the names where the inflate left them
+        rc = idn_gpu_decompress_blocks_ids(w.dev.ctx(), nullptr, off.data(), rb.len.data(), rb.crc.data(), n_blocks, mode, handles.data(),
+                                           (uint32_t)handles.size(), out.acids.data(), out.quals.data(), out.read_off.data(), tot.n_reads,
+                                           tot.n_symbols, &bad);
+    } else {
+        // with identifiers the call is not pipelined and can use the bytes idn_gpu_index_blocks left on the device (blocks == NULL)
+        rc = idn_gpu_decompress_blocks(w.dev.ctx(), out.any_names ? nullptr : rb.base, off.data(), rb.len.data(), rb.crc.data(), n_blocks, mode,
+                                       handles.data(), (uint32_t)handles.size(), out.any_names ? out.names.data() : nullptr,
+                                       out.any_names ? out.name_off.data() : nullptr, out.acids.data(), out.quals.data(), out.read_off.data(),
+                                       tot.n_reads, tot.n_symbols, &bad);
+    }
     if (rc) w.dev.raise(rc);
     out.acids.resize(tot.n_symbols);
     out.quals.resize(tot.n_symbols);
@@ -1177,22 +1213,32 @@ IdnDecompressor::DecodedBatch IdnDecompressor::decode_text(Worker& w, const RawB
                                   block_first.data());
     }
     if (rc) w.dev.raise(rc);
-    {
+    // the names of the device path never leave it
+    uint64_t dev_name_bytes = 0;
+    const bool on_dev = params_.identifiers_on_device && inflate_names_device(w, rb, off, block_first, tot.n_reads, out, false, &dev_name_bytes);
+    if (!on_dev) {
         Span sp(T_NINFLATE);
         inflate_names(rb, off, block_first, tot.n_reads, out);
     }
     Span sp_d(T_DECODE);
     if (out.names.empty()) out.names.push_back(0);
-    const uint64_t name_bytes = out.any_names ? out.name_off[tot.n_reads] : 0;
+    const uint64_t name_bytes = on_dev ? dev_name_bytes : out.any_names ? out.name_off[tot.n_reads] : 0;
     const uint64_t cap = 2 * tot.n_symbols + 6 * tot.n_reads + name_bytes * (title_with_separator ? 2 : 1) + 64;
-    out.text = pool_.get(cap);
     uint64_t text_len = 0, n_reads = 0;
     int32_t bad = -1;
-    // blocks == NULL: the bytes idn_gpu_index_blocks just uploaded are still on the device
-    rc = idn_gpu_decompress_to_fastq(w.dev.ctx(), nullptr, off.data(), rb.len.data(), rb.crc.data(), n_blocks, mode, handles.data(),
-                                     (uint32_t)handles.size(), out.any_names ? out.names.data() : nullptr,
-                                     out.any_names ? out.name_off.data() : nullptr, tot.n_reads, tot.n_symbols, title_with_separator ? 1 : 0,
-                                     out.text->p, cap, &text_len, &n_reads, &bad);
+    if (on_dev) {
+        out.text = pool_.get(cap);
+        rc = idn_gpu_decompress_to_fastq_ids(w.dev.ctx(), nullptr, off.data(), rb.len.data(), rb.crc.data(), n_blocks, mode, handles.data(),
+                                             (uint32_t)handles.size(), tot.n_reads, tot.n_symbols, title_with_separator ? 1 : 0, out.text->p, cap,
+                                             &text_len, &n_reads, &bad);
+    } else {
+        out.text = pool_.get(cap);
+        // blocks == NULL: the bytes idn_gpu_index_blocks just uploaded are still on the device
+        rc = idn_gpu_decompress_to_fastq(w.dev.ctx(), nullptr, off.data(), rb.len.data(), rb.crc.data(), n_blocks, mode, handles.data(),
+                                         (uint32_t)handles.size(), out.any_names ? out.names.data() : nullptr,
+                                         out.any_names ? out.name_off.data() : nullptr, tot.n_reads, tot.n_symbols, title_with_separator ? 1 : 0,
+                                         out.text->p, cap, &text_len, &n_reads, &bad);
+    }
     if (rc) w.dev.raise(rc);
     out.text_len = text_len;
     out.read_off.assign(1, n_reads);  // [0] = sequences in the text

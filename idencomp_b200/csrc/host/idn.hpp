@@ -241,6 +241,9 @@ struct IdnDecompressorParams {
     uint32_t thread_num = 0;
     std::vector<int32_t> devices{0};  // batches of `batch_blocks` blocks go round robin to these GPUs, results come back in order
     uint32_t batch_blocks = 32;
+    // inflate the Identifiers slices on the device (idn_gpu_inflate_names) instead of with zlib on thread_num host threads;
+    // a batch with a Brotli slice falls back to the host
+    bool identifiers_on_device = false;
 };
 
 class IdnDecompressor {
@@ -284,6 +287,9 @@ private:
     bool read_raw(RawBatch& rb);  // false once the terminator block was seen (and rb holds no block)
     DecodedBatch decode_batch(Worker& w, const RawBatch& rb) const;
     DecodedBatch decode_text(Worker& w, const RawBatch& rb, bool title_with_separator) const;  // text in DecodedBatch::acids
+    // identifiers_on_device: idn_gpu_inflate_names of the batch indexed last; false when it holds a Brotli slice
+    bool inflate_names_device(Worker& w, const RawBatch& rb, const std::vector<uint64_t>& off, const std::vector<uint32_t>& block_first,
+                              uint64_t n_reads, DecodedBatch& out, bool fetch, uint64_t* n_name_bytes) const;
     void inflate_names(const RawBatch& rb, const std::vector<uint64_t>& off, const std::vector<uint32_t>& block_first, uint64_t n_reads,
                        DecodedBatch& out) const;
     void prefetch();

@@ -15,6 +15,7 @@
 #include "idn_fastq.cuh"
 #include "idn_native.cuh"
 #include "idn_deflate.cuh"
+#include "idn_inflate.cuh"
 
 using namespace idn;
 
@@ -141,6 +142,14 @@ struct idn_gpu_ctx {
     DevBuf w_bucket, w_list;       // per-read selection: reads bucketed by model pair (cnt | base | cursor, read list)
     // identifiers Deflate (idn_deflate.cuh): per-block tables, joined names, candidates, tokens, segment records, slices
     DevBuf z_blk, z_joined, z_cand, z_tok, z_ntok, z_rec, z_segblock, z_segoff, z_out;
+    // identifiers Inflate (idn_inflate.cuh): streams, chunks, their state and 16-bit output, the joined text, the names
+    DevBuf i_misc, i_streams, i_chunks, i_cs, i_ss, i_scratch, i_text, i_bstream, i_names, i_nameoff;
+    uint32_t inflate_range = idn::inf::kDefaultRange;  // idn_gpu_set_inflate_range
+    double inflate_ratio = 12.0;   // 16-bit scratch entries per compressed byte of a chunk (grows when a call outgrows it)
+    bool names_valid = false;      // the last idn_gpu_inflate_names succeeded: i_names / i_nameoff hold ...
+    uint32_t names_blocks = 0;     // ... the names of that many blocks ...
+    uint64_t names_reads = 0, names_bytes = 0;  // ... and reads, and their size
+    bool names_any = false;        // some block had an Identifiers slice
     bool bucket_pairs = true;      // IDN_NO_BUCKETS=1: the run-time generic kernels over all reads instead (for comparison)
     uint64_t resident_bytes = 0;   // container bytes idn_gpu_index_blocks / the decoder left in s_blocks ...
     uint32_t resident_blocks = 0;  // ... and how many blocks they are (0: nothing a decode call may reuse)
@@ -464,7 +473,8 @@ extern "C" void idn_gpu_destroy(idn_gpu_ctx* ctx) {
                       &ctx->s_nameoff, &ctx->s_out,     &ctx->s_blockoff, &ctx->s_crc,       &ctx->s_stats,  &ctx->s_sizes,
                       &ctx->s_blocks,  &ctx->s_blocklen, &ctx->s_aout,    &ctx->s_qout,    &ctx->s_offout,     &ctx->s_status, &ctx->s_idx,
                       &ctx->z_blk, &ctx->z_joined, &ctx->z_cand, &ctx->z_tok, &ctx->z_ntok, &ctx->z_rec, &ctx->z_segblock,
-                      &ctx->z_segoff, &ctx->z_out};
+                      &ctx->z_segoff, &ctx->z_out, &ctx->i_misc, &ctx->i_streams, &ctx->i_chunks, &ctx->i_cs, &ctx->i_ss,
+                      &ctx->i_scratch, &ctx->i_text, &ctx->i_bstream, &ctx->i_names, &ctx->i_nameoff};
     for (DevBuf* b : bufs) b->release();
     pipe_destroy(ctx->pipe);
     cudaFree(ctx->d_models);
@@ -1809,11 +1819,14 @@ extern "C" int32_t idn_gpu_index_blocks(idn_gpu_ctx* ctx, const uint8_t* blocks,
 static int32_t decompress_to_staging(idn_gpu_ctx* ctx, const uint8_t* blocks, const uint64_t* block_off, const uint32_t* block_len,
                                      const uint32_t* block_crc, uint32_t n_blocks, int32_t mode, const idn_model_t* models,
                                      uint32_t n_models, const uint8_t* names, const uint64_t* name_off, uint64_t out_reads_cap,
-                                     uint64_t out_symbols_cap, uint64_t* R_out, uint64_t* S_out, int32_t* bad_block) {
+                                     uint64_t out_symbols_cap, uint64_t* R_out, uint64_t* S_out, int32_t* bad_block, bool ids = false) {
     if (!ctx) return IDN_E_INVALID_ARG;
     if (bad_block) *bad_block = -1;
     if (!block_off) return fail(ctx, IDN_E_INVALID_ARG, "NULL argument");
     if ((names != nullptr) != (name_off != nullptr)) return fail(ctx, IDN_E_INVALID_ARG, "names and name_off go together");
+    // ids: the names idn_gpu_inflate_names left on the device (i_names / i_nameoff) instead of host ones
+    if (ids && (!ctx->names_valid || ctx->names_blocks != n_blocks))
+        return fail(ctx, IDN_E_INVALID_ARG, "no idn_gpu_inflate_names call of these blocks precedes this call");
     int32_t rc0 = check_block_table(ctx, block_off, block_len, n_blocks);
     if (rc0) return rc0;
     const uint64_t nbytes = n_blocks ? block_off[n_blocks] : 0;
@@ -1839,7 +1852,7 @@ static int32_t decompress_to_staging(idn_gpu_ctx* ctx, const uint8_t* blocks, co
     if (block_len && n_blocks) CU(cudaMemcpyAsync(ctx->s_blocklen.p, block_len, (size_t)n_blocks * 4, cudaMemcpyHostToDevice, st));
     // names join the block CRC (sequence.rs:381-394): when given, the device verifies symbols only and the name bytes are
     // folded in on the host below; otherwise the device compares against the header directly.
-    const bool host_crc = names != nullptr;
+    const bool host_crc = names != nullptr || (ids && ctx->names_any);
     if (block_crc && !host_crc && n_blocks)
         CU(cudaMemcpyAsync(ctx->s_crc.p, block_crc, (size_t)n_blocks * 4, cudaMemcpyHostToDevice, st));
     int32_t rc = idn_gpu_decompress_blocks_dev(ctx, ctx->s_blocks.as<uint8_t>(), ctx->s_blockoff.as<uint64_t>(),
@@ -1864,6 +1877,9 @@ static int32_t decompress_to_staging(idn_gpu_ctx* ctx, const uint8_t* blocks, co
     const uint64_t R = tot[0], S = tot[1];
     *R_out = R;
     *S_out = S;
+    if (ids && R != ctx->names_reads)
+        return fail(ctx, IDN_E_INVALID_ARG, "the blocks hold %llu reads, the inflated names %llu", (unsigned long long)R,
+                    (unsigned long long)ctx->names_reads);
     if (host_crc && n_blocks) {
         // CRC with names on the device: stage names and run the CRC kernels over the decoded batch
         idn_batch d;
@@ -1875,13 +1891,18 @@ static int32_t decompress_to_staging(idn_gpu_ctx* ctx, const uint8_t* blocks, co
         d.quals = ctx->s_qout.as<uint8_t>();
         d.read_off = ctx->s_offout.as<uint64_t>();
         d.block_first_read = ctx->w_readblock.as<uint32_t>();
-        uint64_t nb = R ? name_off[R] : 0;
-        CU(ctx->s_names.ensure(nb + 16));
-        CU(ctx->s_nameoff.ensure((R + 1) * 8));
-        if (nb) CU(cudaMemcpyAsync(ctx->s_names.p, names, nb, cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(ctx->s_nameoff.p, name_off, (R + 1) * 8, cudaMemcpyHostToDevice, st));
-        d.names = ctx->s_names.as<uint8_t>();
-        d.name_off = ctx->s_nameoff.as<uint64_t>();
+        if (ids) {
+            d.names = ctx->i_names.as<uint8_t>();
+            d.name_off = ctx->i_nameoff.as<uint64_t>();
+        } else {
+            uint64_t nb = R ? name_off[R] : 0;
+            CU(ctx->s_names.ensure(nb + 16));
+            CU(ctx->s_nameoff.ensure((R + 1) * 8));
+            if (nb) CU(cudaMemcpyAsync(ctx->s_names.p, names, nb, cudaMemcpyHostToDevice, st));
+            CU(cudaMemcpyAsync(ctx->s_nameoff.p, name_off, (R + 1) * 8, cudaMemcpyHostToDevice, st));
+            d.names = ctx->s_names.as<uint8_t>();
+            d.name_off = ctx->s_nameoff.as<uint64_t>();
+        }
         if (!block_crc) {
             CU(sync_stream(ctx, st));
             return IDN_OK;
@@ -1910,6 +1931,12 @@ extern "C" int32_t idn_gpu_set_pipeline_blocks(idn_gpu_ctx* ctx, uint32_t blocks
     return IDN_OK;
 }
 
+static int32_t decompress_blocks_staged(idn_gpu_ctx* ctx, const uint8_t* blocks, const uint64_t* block_off, const uint32_t* block_len,
+                                        const uint32_t* block_crc, uint32_t n_blocks, int32_t mode, const idn_model_t* models,
+                                        uint32_t n_models, const uint8_t* names, const uint64_t* name_off, uint8_t* acids_out,
+                                        uint8_t* quals_out, uint64_t* read_off_out, uint64_t out_reads_cap, uint64_t out_symbols_cap,
+                                        int32_t* bad_block, bool ids);
+
 extern "C" int32_t idn_gpu_decompress_blocks(idn_gpu_ctx* ctx, const uint8_t* blocks, const uint64_t* block_off,
                                              const uint32_t* block_len, const uint32_t* block_crc, uint32_t n_blocks, int32_t mode,
                                              const idn_model_t* models, uint32_t n_models, const uint8_t* names,
@@ -1924,7 +1951,6 @@ extern "C" int32_t idn_gpu_decompress_blocks(idn_gpu_ctx* ctx, const uint8_t* bl
     int32_t rc0 = check_block_table(ctx, block_off, block_len, n_blocks);
     if (rc0) return rc0;
     CU(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
     if (!names && n_blocks && blocks) {
         // no names on the device (the block CRCs cover the symbols only): sub-chunks of whole blocks flow through upload /
         // kernels / download streams; a sub-chunk that outgrows its share of the staging sends the call down the path below
@@ -1936,9 +1962,20 @@ extern "C" int32_t idn_gpu_decompress_blocks(idn_gpu_ctx* ctx, const uint8_t* bl
                                                   quals_out, read_off_out, out_reads_cap, out_symbols_cap, bad_block, &retry_simple);
         if (rcp || !retry_simple) return rcp;
     }
+    return decompress_blocks_staged(ctx, blocks, block_off, block_len, block_crc, n_blocks, mode, models, n_models, names, name_off, acids_out,
+                                    quals_out, read_off_out, out_reads_cap, out_symbols_cap, bad_block, false);
+}
+
+// the unpipelined decode of idn_gpu_decompress_blocks(_ids) with its results copied to the caller's buffers
+static int32_t decompress_blocks_staged(idn_gpu_ctx* ctx, const uint8_t* blocks, const uint64_t* block_off, const uint32_t* block_len,
+                                        const uint32_t* block_crc, uint32_t n_blocks, int32_t mode, const idn_model_t* models,
+                                        uint32_t n_models, const uint8_t* names, const uint64_t* name_off, uint8_t* acids_out,
+                                        uint8_t* quals_out, uint64_t* read_off_out, uint64_t out_reads_cap, uint64_t out_symbols_cap,
+                                        int32_t* bad_block, bool ids) {
+    cudaStream_t st = ctx->stream;
     uint64_t R = 0, S = 0;
     int32_t rc = decompress_to_staging(ctx, blocks, block_off, block_len, block_crc, n_blocks, mode, models, n_models, names, name_off,
-                                       out_reads_cap, out_symbols_cap, &R, &S, bad_block);
+                                       out_reads_cap, out_symbols_cap, &R, &S, bad_block, ids);
     if (rc) return rc;
     if (S) {
         CU(cudaMemcpyAsync(acids_out, ctx->s_aout.p, S, cudaMemcpyDeviceToHost, st));

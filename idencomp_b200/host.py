@@ -28,7 +28,17 @@ EXPORTS = [
     "idn_host_xoshiro256pp", "idn_host_sample_indices", "idn_host_gen_range", "idn_host_compressor_add_text", "idn_host_decompress_text",
     "idn_host_text_free", "idn_host_decompress_text_into", "idn_host_compressor_set_output",
     "idn_host_release_cached", "idn_host_text_reader_new", "idn_host_text_reader_next", "idn_host_text_reader_free",
+    "idn_host_decompress_ex", "idn_host_decompress_text_ex", "idn_host_decompress_text_into_ex", "idn_host_text_reader_new_ex",
 ]
+
+
+class DecompressParams(C.Structure):
+    """idn_host_decompress_params: the IdnDecompressorParams the _ex entry points take"""
+    _fields_ = [("identifiers_on_device", C.c_int32)]
+
+
+def _dparams(identifiers_on_device: bool):
+    return C.byref(DecompressParams(int(bool(identifiers_on_device))))
 
 
 class Params(C.Structure):
@@ -95,6 +105,11 @@ def load():
     L.idn_host_compressor_free.argtypes = [vp]
     L.idn_host_compressor_free.restype = None
     L.idn_host_decompress.argtypes = [vp, u32, i32, u32, vp, u64, C.POINTER(vp)]
+    L.idn_host_decompress_ex.argtypes = [vp, u32, i32, u32, vp, u64, C.POINTER(vp), C.POINTER(DecompressParams)]
+    L.idn_host_decompress_text_ex.argtypes = [vp, u32, i32, u32, u32, i32, vp, u64, C.POINTER(vp), C.POINTER(u64), C.POINTER(DecompressParams)]
+    L.idn_host_decompress_text_into_ex.argtypes = [vp, u32, i32, u32, u32, i32, vp, u64, vp, u64, C.POINTER(u64), C.POINTER(DecompressParams)]
+    L.idn_host_text_reader_new_ex.argtypes = [vp, u32, C.POINTER(i32), u32, u32, u32, i32, vp, u64, C.POINTER(vp),
+                                              C.POINTER(DecompressParams)]
     for name, rt in (("reads", u64), ("version", u32), ("read_off", vp), ("acids", vp), ("quals", vp), ("name_off", vp), ("names", vp)):
         f = getattr(L, "idn_host_decoded_" + name)
         f.argtypes = [vp]
@@ -322,17 +337,18 @@ class IdnCompressor:
             pass
 
 
-def decompress(models, idn: bytes, *, device=0, n_devices=0, batch_blocks=32) -> dict:
+def decompress(models, idn: bytes, *, device=0, n_devices=0, batch_blocks=32, identifiers_on_device=False) -> dict:
     """idencomp::IdnDecompressor (idn/decompressor.rs:455-566): every sequence of the file as one SoA batch.
-    n_devices > 1: the first n_devices GPUs share the file."""
+    n_devices > 1: the first n_devices GPUs share the file.  identifiers_on_device: the Identifiers slices are inflated on
+    the device (Brotli slices still on the host); the result does not change."""
     if n_devices > 1:
         device = -n_devices
     L = load()
     buf = np.frombuffer(idn, dtype=np.uint8)
     h = C.c_void_p()
     models = list(models)
-    _check(L.idn_host_decompress(_model_array(models), len(models), device, batch_blocks, buf.ctypes.data if buf.size else None,
-                                 buf.size, C.byref(h)))
+    _check(L.idn_host_decompress_ex(_model_array(models), len(models), device, batch_blocks, buf.ctypes.data if buf.size else None,
+                                    buf.size, C.byref(h), _dparams(identifiers_on_device)))
     try:
         n = int(L.idn_host_decoded_reads(h))
         ro = np.ctypeslib.as_array(C.cast(L.idn_host_decoded_read_off(h), C.POINTER(C.c_uint64)), (n + 1,)).copy()
@@ -345,16 +361,19 @@ def decompress(models, idn: bytes, *, device=0, n_devices=0, batch_blocks=32) ->
         L.idn_host_decoded_free(h)
 
 
-def decompress_text(models, idn, *, device=0, n_devices=0, batch_blocks=32, thread_num=0, title_with_separator=False, as_view=False):
-    """IdnDecompressor + FastqWriter (fastq/writer.rs:190-245): the whole file as FASTQ text, formatted on the device."""
+def decompress_text(models, idn, *, device=0, n_devices=0, batch_blocks=32, thread_num=0, title_with_separator=False, as_view=False,
+                    identifiers_on_device=False):
+    """IdnDecompressor + FastqWriter (fastq/writer.rs:190-245): the whole file as FASTQ text, formatted on the device.
+    identifiers_on_device: the names are inflated on the device too and never cross to the host."""
     L = load()
     buf = np.frombuffer(idn, dtype=np.uint8) if isinstance(idn, (bytes, bytearray, memoryview)) else np.ascontiguousarray(idn, dtype=np.uint8)
     models = list(models)
     if n_devices > 1:
         device = -n_devices
     ptr, n = C.c_void_p(), C.c_uint64(0)
-    _check(L.idn_host_decompress_text(_model_array(models), len(models), device, batch_blocks, thread_num, int(title_with_separator),
-                                      buf.ctypes.data if buf.size else None, buf.size, C.byref(ptr), C.byref(n)))
+    _check(L.idn_host_decompress_text_ex(_model_array(models), len(models), device, batch_blocks, thread_num, int(title_with_separator),
+                                         buf.ctypes.data if buf.size else None, buf.size, C.byref(ptr), C.byref(n),
+                                         _dparams(identifiers_on_device)))
     if as_view:  # (view, free): no copy of the text; call free() when done with the view
         view = np.ctypeslib.as_array(C.cast(ptr, C.POINTER(C.c_uint8)), (n.value,)) if n.value else np.zeros(0, dtype=np.uint8)
         return view, (lambda: L.idn_host_text_free(ptr))
@@ -364,7 +383,8 @@ def decompress_text(models, idn, *, device=0, n_devices=0, batch_blocks=32, thre
         L.idn_host_text_free(ptr)
 
 
-def decompress_text_into(models, idn, out: np.ndarray, *, device=0, n_devices=0, batch_blocks=32, thread_num=0, title_with_separator=False) -> int:
+def decompress_text_into(models, idn, out: np.ndarray, *, device=0, n_devices=0, batch_blocks=32, thread_num=0, title_with_separator=False,
+                         identifiers_on_device=False) -> int:
     """decompress_text into the caller's uint8 array (e.g. page-locked); returns the length of the text"""
     L = load()
     buf = np.frombuffer(idn, dtype=np.uint8) if isinstance(idn, (bytes, bytearray, memoryview)) else np.ascontiguousarray(idn, dtype=np.uint8)
@@ -372,8 +392,9 @@ def decompress_text_into(models, idn, out: np.ndarray, *, device=0, n_devices=0,
     if n_devices > 1:
         device = -n_devices
     n = C.c_uint64(0)
-    _check(L.idn_host_decompress_text_into(_model_array(models), len(models), device, batch_blocks, thread_num, int(title_with_separator),
-                                           buf.ctypes.data if buf.size else None, buf.size, out.ctypes.data, out.size, C.byref(n)))
+    _check(L.idn_host_decompress_text_into_ex(_model_array(models), len(models), device, batch_blocks, thread_num, int(title_with_separator),
+                                              buf.ctypes.data if buf.size else None, buf.size, out.ctypes.data, out.size, C.byref(n),
+                                              _dparams(identifiers_on_device)))
     return int(n.value)
 
 
@@ -386,16 +407,16 @@ class FastqTextReader:
     """streaming text out: iterating yields the FASTQ text of one batch of blocks at a time as a uint8 view of the library's
     page-locked memory (valid until the next step) -- what a writer would hand to write()"""
 
-    def __init__(self, models, idn, *, devices=(0,), batch_blocks=32, thread_num=0, title_with_separator=False):
+    def __init__(self, models, idn, *, devices=(0,), batch_blocks=32, thread_num=0, title_with_separator=False, identifiers_on_device=False):
         self.L = load()
         self._idn = np.frombuffer(idn, dtype=np.uint8) if isinstance(idn, (bytes, bytearray, memoryview)) else np.ascontiguousarray(idn, dtype=np.uint8)
         models = list(models)
         self._models = models
         devs = (C.c_int32 * max(1, len(devices)))(*devices)
         h = C.c_void_p()
-        _check(self.L.idn_host_text_reader_new(_model_array(models), len(models), devs, len(devices), batch_blocks, thread_num,
-                                               int(title_with_separator), self._idn.ctypes.data if self._idn.size else None, self._idn.size,
-                                               C.byref(h)))
+        _check(self.L.idn_host_text_reader_new_ex(_model_array(models), len(models), devs, len(devices), batch_blocks, thread_num,
+                                                  int(title_with_separator), self._idn.ctypes.data if self._idn.size else None, self._idn.size,
+                                                  C.byref(h), _dparams(identifiers_on_device)))
         self.h = h
 
     def __iter__(self):

@@ -316,6 +316,44 @@ int32_t idn_gpu_deflate_names_dev(idn_gpu_ctx *ctx, const uint8_t *names, const 
 /* upper bound of slice_off[n_blocks] for any names of this shape (name_bytes = name_off[R] - name_off[0]) */
 uint64_t idn_gpu_deflate_names_bound(uint64_t name_bytes, uint64_t n_reads, uint32_t n_blocks);
 
+/* ---- identifiers slices: raw Inflate (RFC 1951) on the device ----------------------------------------------------------
+ * What the host's inflate_names does for a batch of blocks (decompressor_block.rs:146-192), on the device: every block's
+ * leading Identifiers slices (0x00 | u32be n | compression | n bytes) are inflated, joined with '\n', and split at '\n'
+ * into at most as many names as the block has reads (block b holds reads [block_first_read[b], block_first_read[b+1]));
+ * reads without a line get an empty name, text after the last wanted line is dropped.  Acceptance is zlib's raw inflate
+ * (windowBits -15), bytes after the final block included.  blocks / block_off / block_len are as idn_gpu_decompress_blocks
+ * takes them; blocks == NULL uses the bytes the last idn_gpu_index_blocks call left on the device (same rule as the decode
+ * calls) and keeps them there.  The names stay in the ctx: idn_gpu_inflate_names_fetch copies them out (names:
+ * n_name_bytes bytes, name_off: n_reads + 1 entries), the _ids decode calls below read them where they are.
+ * IDN_E_UNSUPPORTED for a Brotli slice (compression 0; nothing is written), IDN_E_SERIALIZE for a compression byte above 1,
+ * a truncated slice or a slice that does not inflate, with bad_block = the first such block. */
+typedef struct {
+    uint64_t n_streams;     /* Identifiers slices (0: no block has names) */
+    uint64_t n_chunks;      /* ranges the slices were cut into (idn_gpu_set_inflate_range) */
+    uint64_t n_speculative; /* chunks after a slice's first that found a block start and were decoded from it */
+    uint64_t n_joined;      /* of them, chunks whose start the verified decode before them ended on */
+    uint64_t serial_bytes;  /* output bytes decoded again from the end of the verified decode (chunks that did not join) */
+    uint64_t in_bytes;      /* Deflate bytes of all slices */
+} idn_inflate_stats;
+
+int32_t idn_gpu_inflate_names(idn_gpu_ctx *ctx, const uint8_t *blocks, const uint64_t *block_off, const uint32_t *block_len /* optional */,
+                              uint32_t n_blocks, const uint32_t *block_first_read /*[n_blocks+1]*/, uint64_t n_reads,
+                              uint64_t *n_name_bytes, int32_t *bad_block, idn_inflate_stats *stats /* optional */);
+int32_t idn_gpu_inflate_names_fetch(idn_gpu_ctx *ctx, uint8_t *names, uint64_t *name_off);
+/* compressed bytes per range of the parallel inflate (default 4096); results do not depend on it */
+int32_t idn_gpu_set_inflate_range(idn_gpu_ctx *ctx, uint32_t bytes);
+/* idn_gpu_decompress_blocks / idn_gpu_decompress_to_fastq with the names the preceding idn_gpu_inflate_names call on this
+ * ctx left on the device, for the block CRC and the title lines (no host round trip; the calls are not pipelined).
+ * IDN_E_INVALID_ARG without such a call of the same number of blocks and reads. */
+int32_t idn_gpu_decompress_blocks_ids(idn_gpu_ctx *ctx, const uint8_t *blocks, const uint64_t *block_off,
+                                      const uint32_t *block_len /* optional */, const uint32_t *block_crc, uint32_t n_blocks, int32_t mode,
+                                      const idn_model_t *models, uint32_t n_models, uint8_t *acids_out, uint8_t *quals_out,
+                                      uint64_t *read_off_out, uint64_t out_reads_cap, uint64_t out_symbols_cap, int32_t *bad_block);
+int32_t idn_gpu_decompress_to_fastq_ids(idn_gpu_ctx *ctx, const uint8_t *blocks, const uint64_t *block_off, const uint32_t *block_len,
+                                        const uint32_t *block_crc, uint32_t n_blocks, int32_t mode, const idn_model_t *models,
+                                        uint32_t n_models, uint64_t reads_cap, uint64_t symbols_cap, int32_t title_with_separator,
+                                        uint8_t *text, uint64_t text_cap, uint64_t *text_len, uint64_t *n_reads_out, int32_t *bad_block);
+
 /* ---- per-kernel timing (CUDA events on the launching stream; what bench.py's roofline line is made of) ----
  * idn_gpu_profile(ctx, 1) starts recording an event after every kernel launch of the *_dev entry points;
  * idn_gpu_profile_read synchronises the device and writes one text line per kernel, "name launches total_ms",

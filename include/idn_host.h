@@ -131,6 +131,24 @@ const uint8_t *idn_host_decoded_quals(const idn_host_decoded *d);
 const uint64_t *idn_host_decoded_name_off(const idn_host_decoded *d); /* [reads+1] */
 const uint8_t *idn_host_decoded_names(const idn_host_decoded *d);
 void idn_host_decoded_free(idn_host_decoded *d);
+/* decompressor parameters the forms above leave at their defaults (IdnDecompressorParams) */
+typedef struct {
+    int32_t identifiers_on_device; /* inflate the Identifiers slices on the device (idn_gpu_inflate_names); default 0 */
+} idn_host_decompress_params;
+/* the decompression entry points with parameters (NULL = the defaults, which is what the forms without _ex use) */
+int32_t idn_host_decompress_ex(const idn_host_model *const *models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
+                               const uint8_t *idn, uint64_t idn_len, idn_host_decoded **out, const idn_host_decompress_params *dparams);
+int32_t idn_host_decompress_text_ex(const idn_host_model *const *models, uint32_t n_models, int32_t device, uint32_t batch_blocks,
+                                    uint32_t thread_num, int32_t title_with_separator, const uint8_t *idn, uint64_t idn_len,
+                                    uint8_t **text, uint64_t *text_len, const idn_host_decompress_params *dparams);
+int32_t idn_host_decompress_text_into_ex(const idn_host_model *const *models, uint32_t n_models, int32_t device,
+                                         uint32_t batch_blocks, uint32_t thread_num, int32_t title_with_separator,
+                                         const uint8_t *idn, uint64_t idn_len, uint8_t *text, uint64_t cap, uint64_t *text_len,
+                                         const idn_host_decompress_params *dparams);
+int32_t idn_host_text_reader_new_ex(const idn_host_model *const *models, uint32_t n_models, const int32_t *devices,
+                                    uint32_t n_devices, uint32_t batch_blocks, uint32_t thread_num, int32_t title_with_separator,
+                                    const uint8_t *idn, uint64_t idn_len, idn_host_text_reader **out,
+                                    const idn_host_decompress_params *dparams);
 
 /* ---- file-level model subset selection on a cost matrix cost[value][centroid] (exposed for the known-answer tests) ----
  * Clustering::make_clusters (clustering.rs:21-118): centroid index per cluster and the cluster of every value;
