@@ -753,7 +753,11 @@ size_t IdnCompressor::consume_text(const uint8_t* buf, size_t total, bool final)
         int32_t rc = idn_gpu_fastq_parse_chunk(w->dev.ctx(), buf + text_pos_, len, last ? 1 : 0, params_.max_block_total_len, &ck);
         if (rc) {
             std::string what = idn_gpu_last_error(w->dev.ctx());
-            if (ck.error_kind) what = std::string("FastqReaderError::") + fastq_error_name(ck.error_kind) + ": " + what;
+            if (ck.error_kind) {  // the chunk counts records from its own start; the caller wants them from the file's
+                char rec[64];
+                snprintf(rec, sizeof rec, " at record %llu", (unsigned long long)(stats_.in_reads + ck.bad_record));
+                what = std::string("FastqReaderError::") + fastq_error_name(ck.error_kind) + rec;
+            }
             if (rc == IDN_E_CUDA) w->dev.mark_broken();
             w->release();
             throw IdnError(rc, what);

@@ -9,7 +9,7 @@
 // parse_title does), then one thread per record validates and converts.  Same acceptance rules as the reference:
 // the title starts with '@' and is trimmed, acids are ATCGN, the separator line starts with '+', quality scores are
 // '!'..'~', both symbol lines have one length, a record that ends early is an error.  (Rust's trim() also strips
-// non-ASCII Unicode white space; here ASCII white space only.)
+// non-ASCII Unicode white space; here ASCII white space only.)  The reader reports the first error in file order.
 #pragma once
 #include "idn_kernels.cuh"
 
@@ -205,7 +205,8 @@ struct FastqView {
     uint64_t n_reads;
 };
 
-// per record: trimmed name span and symbol count; structural errors (no '@', record cut short)
+// per record: trimmed name span and symbol count; a title without '@'.  Every other check is fq_convert_kernel's, so
+// that a record's checks run in the reference's order and the lowest record wins the atomicMin.
 __global__ void __launch_bounds__(128)
 fq_lengths_kernel(FastqView V, unsigned long long* __restrict__ name_lo, uint32_t* __restrict__ name_len,
                   uint32_t* __restrict__ read_len, unsigned long long* __restrict__ first_err) {
@@ -221,11 +222,8 @@ fq_lengths_kernel(FastqView V, unsigned long long* __restrict__ name_lo, uint32_
     name_lo[r] = lo;
     name_len[r] = err ? 0 : (uint32_t)(hi - lo);
     uint32_t len = 0;
-    if (t + 3 >= V.n_lines) {
-        if (!err) err = kFqEof;  // EofReached inside a record
-    } else {
+    if (t + 3 < V.n_lines)  // a record cut short is fq_convert_kernel's to report
         len = (uint32_t)(fq_line_end(V.line_start, t + 1, V.n_lines, V.n_newlines, V.n) - V.line_start[t + 1]);
-    }
     read_len[r] = len;
     if (err) atomicMin(first_err, (r << 8) | err);
 }
@@ -235,7 +233,24 @@ struct U32Fn {
     __device__ __forceinline__ unsigned long long operator()(uint64_t i) const { return v[i]; }
 };
 
-// per record: name bytes, acids and quality scores through the reference's byte tables
+// The last record, cut short at the end of the text: the lines it has are checked in the reference's order before
+// EofReached.  Only its error matters, so nothing is written.  Kept out of line so that it costs fq_convert_kernel no
+// registers.
+__device__ __noinline__ uint32_t fq_cut_short_err(FastqView V, uint64_t t) {
+    if (t + 1 >= V.n_lines) return kFqEof;
+    const unsigned long long a_lo = V.line_start[t + 1], a_hi = fq_line_end(V.line_start, t + 1, V.n_lines, V.n_newlines, V.n);
+    for (unsigned long long p = a_lo; p < a_hi; p++) {
+        const uint8_t c = V.text[p];
+        if (c != 'A' && c != 'C' && c != 'T' && c != 'G' && c != 'N') return kFqInvalidAcid;
+    }
+    if (t + 2 >= V.n_lines) return kFqEof;
+    const unsigned long long s_lo = V.line_start[t + 2], s_hi = fq_line_end(V.line_start, t + 2, V.n_lines, V.n_newlines, V.n);
+    if (s_hi == s_lo || V.text[s_lo] != '+') return kFqInvalidFormat;
+    return kFqEof;
+}
+
+// per record: name bytes, acids and quality scores through the reference's byte tables.  The checks run in the
+// reference's order: acids, the separator, every byte of the quality line, then the lengths.
 __global__ void __launch_bounds__(128)
 fq_convert_kernel(FastqView V, const unsigned long long* __restrict__ name_lo, const unsigned long long* __restrict__ name_off,
                   const unsigned long long* __restrict__ read_off, uint8_t* __restrict__ names, uint8_t* __restrict__ acids,
@@ -243,7 +258,10 @@ fq_convert_kernel(FastqView V, const unsigned long long* __restrict__ name_lo, c
     uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= V.n_reads) return;
     const uint64_t t = V.title_line[r];
-    if (t + 3 >= V.n_lines) return;  // reported by fq_lengths_kernel
+    if (t + 3 >= V.n_lines) {
+        atomicMin(first_err, (r << 8) | fq_cut_short_err(V, t));
+        return;
+    }
     const uint32_t nl = (uint32_t)(name_off[r + 1] - name_off[r]);
     for (uint32_t i = 0; i < nl; i++) names[name_off[r] + i] = V.text[name_lo[r] + i];
     const unsigned long long a_lo = V.line_start[t + 1], a_hi = fq_line_end(V.line_start, t + 1, V.n_lines, V.n_newlines, V.n);

@@ -2256,11 +2256,10 @@ static int32_t fastq_parse_dev_impl(idn_gpu_ctx* ctx, const uint8_t* text, uint6
     unsigned long long tot[2] = {0, 0}, ferr = ~0ull;
     CU(cudaMemcpyAsync(&tot[0], read_off + n_reads, 8, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(&tot[1], name_off + n_reads, 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ferr, first_err, 8, cudaMemcpyDeviceToHost, st));
     CU(sync_stream(ctx, st));
     info->n_symbols = tot[0];
     info->n_name_bytes = tot[1];
-    if (ferr == ~0ull && n_reads) {
+    if (n_reads) {  // also after a title without '@': an earlier record may hold an earlier error
         CU(ctx->f_names.ensure(tot[1] + 16));
         CU(ctx->f_acids.ensure(tot[0] + 16));
         CU(ctx->f_quals.ensure(tot[0] + 16));

@@ -233,7 +233,8 @@ int32_t idn_gpu_synth_reads_dev(idn_gpu_ctx *ctx, idn_model_t acid_model, idn_mo
  * is expected, the title starts with '@' and is trimmed, acids are ATCGN, the separator line starts with '+', quality
  * scores are '!'..'~', both symbol lines have one length.  A violation fails with IDN_E_SERIALIZE; error_kind names
  * the FastqReaderError variant (1 InvalidFormat, 2 InvalidAcid, 3 InvalidQualityScore, 4 length mismatch, 5 end of
- * input inside a record) and bad_record the first offending record. */
+ * input inside a record) and bad_record the record, counted from 0, that the reference stops at: the first error in
+ * file order, a record's lines checked in the reference's order. */
 typedef struct {
     uint64_t n_reads, n_symbols, n_name_bytes, n_lines;
     int32_t error_kind;

@@ -1092,7 +1092,16 @@ int orc_decompress(const orc_model_t *const *models, uint32_t n_models, const ui
 
 /* ------------------------------------------------------------------------------------------------
  * FASTQ text (fastq/reader.rs:166-282, consts.rs:28-98, writer.rs:190-240) -- host-side, out of the GPU
- * path; here so the goldens (samples/*.fastq) can be turned into symbol arrays.
+ * path; here so the goldens (samples/*.fastq) can be turned into symbol arrays, and as the statement the
+ * device reader's acceptance and error reports are checked against.
+ *
+ * A record is checked in the reference's order: the title starts with '@' (untrimmed line), the acids
+ * line is present, every acid is valid, the separator line is present and starts with '+', the quality
+ * line is present, every byte of the whole quality line is valid, and only then are the two lengths
+ * compared.  A missing line is EofReached.  Blank lines (ASCII white space only: 0x09-0x0D and ' ', as
+ * str::trim does for ASCII) are skipped where a title is expected, and the title is trimmed with the same
+ * set.  A failure is reported as "FastqReaderError::<variant> at record <r>", r counted from 0 in file
+ * order; oracle.py parses that form.
  * ---------------------------------------------------------------------------------------------- */
 static const uint8_t *next_line(const uint8_t *p, const uint8_t *end, const uint8_t **ls, const uint8_t **le) {
     if (p >= end) return NULL;
@@ -1100,6 +1109,12 @@ static const uint8_t *next_line(const uint8_t *p, const uint8_t *end, const uint
     *ls = p;
     *le = nl ? nl : end;
     return nl ? nl + 1 : end;
+}
+
+static int fq_ws(uint8_t c) { return c == ' ' || (c >= 9 && c <= 13); }
+
+static int fq_fail(const char *variant, uint64_t record) {
+    return fail(ORC_E_FASTQ, "FastqReaderError::%s at record %llu", variant, (unsigned long long)record);
 }
 
 int orc_fastq_parse(const uint8_t *text, size_t n, orc_decoded_t *out) {
@@ -1111,60 +1126,60 @@ int orc_fastq_parse(const uint8_t *text, size_t n, orc_decoded_t *out) {
     const uint8_t *p = text, *end = text + n, *ls, *le;
     int rc = ORC_OK;
     for (;;) {
+        const uint64_t rec = out->n_reads;
         /* parse_title: skip blank lines, require '@', trim */
         const uint8_t *q;
         int got = 0;
         while ((q = next_line(p, end, &ls, &le)) != NULL) {
             p = q;
             const uint8_t *a = ls, *b = le;
-            while (a < b && (*a == ' ' || *a == '\t' || *a == '\r')) a++;
-            while (b > a && (b[-1] == ' ' || b[-1] == '\t' || b[-1] == '\r')) b--;
+            while (a < b && fq_ws(*a)) a++;
             if (a < b) {
                 got = 1;
                 break;
             }
         }
         if (!got) break; /* EOF */
-        if (*ls != '@') { rc = fail(ORC_E_FASTQ, "invalid FASTQ title line"); break; }
+        if (*ls != '@') { rc = fq_fail("InvalidFormat", rec); break; }
         const uint8_t *a = ls + 1, *b = le;
-        while (a < b && (*a == ' ' || *a == '\t' || *a == '\r')) a++;
-        while (b > a && (b[-1] == ' ' || b[-1] == '\t' || b[-1] == '\r')) b--;
+        while (a < b && fq_ws(*a)) a++;
+        while (b > a && fq_ws(b[-1])) b--;
         buf_put(&nm, a, (size_t)(b - a));
         /* acids */
-        if ((q = next_line(p, end, &ls, &le)) == NULL) { rc = fail(ORC_E_FASTQ, "EOF in record"); break; }
+        if ((q = next_line(p, end, &ls, &le)) == NULL) { rc = fq_fail("EofReached", rec); break; }
         p = q;
         size_t alen = (size_t)(le - ls);
         buf_reserve(&ac, alen);
-        for (size_t i = 0; i < alen; i++) {
-            uint8_t ch = ls[i], v;
-            switch (ch) { /* Acid repr: N=0 A=1 C=2 T=3 G=4  sequence.rs:401-413 */
+        for (size_t i = 0; i < alen && !rc; i++) {
+            uint8_t v;
+            switch (ls[i]) { /* Acid repr: N=0 A=1 C=2 T=3 G=4  sequence.rs:401-413 */
             case 'N': v = 0; break;
             case 'A': v = 1; break;
             case 'C': v = 2; break;
             case 'T': v = 3; break;
             case 'G': v = 4; break;
-            default: rc = fail(ORC_E_FASTQ, "invalid acid '%c'", ch); v = 0;
+            default: rc = fq_fail("InvalidAcid", rec); v = 0;
             }
             ac.data[ac.len + i] = v;
         }
         if (rc) break;
         ac.len += alen;
         /* separator */
-        if ((q = next_line(p, end, &ls, &le)) == NULL) { rc = fail(ORC_E_FASTQ, "EOF in record"); break; }
+        if ((q = next_line(p, end, &ls, &le)) == NULL) { rc = fq_fail("EofReached", rec); break; }
         p = q;
-        if (le == ls || *ls != '+') { rc = fail(ORC_E_FASTQ, "invalid separator line"); break; }
-        /* quality */
-        if ((q = next_line(p, end, &ls, &le)) == NULL) { rc = fail(ORC_E_FASTQ, "EOF in record"); break; }
+        if (le == ls || *ls != '+') { rc = fq_fail("InvalidFormat", rec); break; }
+        /* quality scores: the whole line is converted before the lengths are compared */
+        if ((q = next_line(p, end, &ls, &le)) == NULL) { rc = fq_fail("EofReached", rec); break; }
         p = q;
         size_t qlen = (size_t)(le - ls);
-        if (qlen != alen) { rc = fail(ORC_E_FASTQ, "acid/quality length mismatch"); break; }
         buf_reserve(&qu, qlen);
         for (size_t i = 0; i < qlen; i++) {
             uint8_t ch = ls[i];
-            if (ch < '!' || ch > '~') { rc = fail(ORC_E_FASTQ, "invalid quality score byte %u", ch); break; }
+            if (ch < '!' || ch > '~') { rc = fq_fail("InvalidQualityScore", rec); break; }
             qu.data[qu.len + i] = (uint8_t)(ch - '!');
         }
         if (rc) break;
+        if (qlen != alen) { rc = fq_fail("AcidAndQualityScoreLengthMismatch", rec); break; }
         qu.len += qlen;
         uint64_t t = ac.len, nn = nm.len;
         buf_put(&ro, &t, 8);

@@ -13,6 +13,7 @@ from __future__ import annotations
 import ctypes as C
 import hashlib
 import os
+import re
 import struct
 import subprocess
 from dataclasses import dataclass
@@ -392,9 +393,20 @@ def _take_decoded(d: _Decoded) -> Reads:
 
 
 def fastq_parse(text: bytes) -> Reads:
+    """FastqReader::read_sequence until EOF (fastq/reader.rs:166-282).  On malformed input raises OracleError
+    (FastqError) with .fastq_error = the FastqReaderError variant (as capi.FASTQ_ERRORS names it) and .bad_record =
+    the 0-based record, in file order, that the reference stops at."""
     t = np.frombuffer(text, dtype=np.uint8)
     d = _Decoded()
-    _check(lib().orc_fastq_parse(_ptr(t), len(t), C.byref(d)))
+    rc = lib().orc_fastq_parse(_ptr(t), len(t), C.byref(d))
+    if rc != 0:
+        msg = lib().orc_last_error().decode()
+        e = OracleError(rc, msg)
+        m = re.fullmatch(r"FastqReaderError::(\w+) at record (\d+)", msg)
+        if m is None:
+            raise e
+        e.fastq_error, e.bad_record = m.group(1), int(m.group(2))
+        raise e
     try:
         return _take_decoded(d)
     finally:
