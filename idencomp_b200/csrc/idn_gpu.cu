@@ -1027,10 +1027,19 @@ extern "C" int32_t idn_gpu_compress_blocks_dev(idn_gpu_ctx* ctx, const idn_batch
         CU(cudaMemsetAsync(slice_off, 0, 8, st));
     }
     CU(ctx->w_blockadj.ensure(((size_t)B + 1) * 8));
-    block_layout_kernel<<<1, 32, 0, st>>>(slice_off, batch->block_first_read, B, prefix_len, fast,
-                                          reinterpret_cast<unsigned long long*>(block_off), out, out_cap, dsp->stats,
-                                          ctx->w_blockadj.as<unsigned long long>());
-    LAUNCHED("block_layout");
+    {  // block layout: sizes, their exclusive scan, then the headers (all three timed as "block_layout")
+        unsigned long long* boff = reinterpret_cast<unsigned long long*>(block_off);
+        const unsigned lgrid = (unsigned)((B + 255) / 256);
+        if (B) {
+            block_size_kernel<<<lgrid, 256, 0, st>>>(slice_off, batch->block_first_read, B, prefix_len, fast, boff);
+            LAUNCHED("block_layout");
+        }
+        scan_tiles_kernel<<<1, kScanBlock, 0, st>>>(boff, B);
+        LAUNCHED("block_layout");
+        block_layout_kernel<<<lgrid ? lgrid : 1, 256, 0, st>>>(slice_off, batch->block_first_read, B, prefix_len, fast, boff, out,
+                                                             out_cap, dsp->stats, ctx->w_blockadj.as<unsigned long long>());
+        LAUNCHED("block_layout");
+    }
     if (R > 0) {
         read_block_kernel<<<B, 256, 0, st>>>(batch->block_first_read, B, ctx->w_readblock.as<uint32_t>());
         LAUNCHED("read_block");
@@ -1047,7 +1056,8 @@ extern "C" int32_t idn_gpu_compress_blocks_dev(idn_gpu_ctx* ctx, const idn_batch
         aa.cand_index = dsp->cand_index;
         aa.out = out;
         aa.out_cap = out_cap;
-        assemble_kernel<<<(unsigned)((R + 127) / 128), 128, 0, st>>>(aa);
+        aa.lanes_log2 = assemble_lanes_log2(S, R);
+        assemble_kernel<<<(unsigned)(((R << aa.lanes_log2) + kAssembleBlock - 1) / kAssembleBlock), kAssembleBlock, 0, st>>>(aa);
         LAUNCHED("assemble");
         stats_kernel<<<592, 256, 0, st>>>(ctx->w_paylen.as<uint32_t>(), switched, R, dsp->stats);
         LAUNCHED("stats");

@@ -891,41 +891,51 @@ struct SliceSize {
     }
 };
 
-// one thread per block: block_base[b] = absolute offset of block b's header in `out`
-// (sequential over blocks inside one thread block of 1 warp; n_blocks is small -- hundreds)
-__global__ void __launch_bounds__(32)
-block_layout_kernel(const unsigned long long* __restrict__ slice_off, const uint32_t* __restrict__ block_first,
-                    uint32_t n_blocks, const uint32_t* __restrict__ prefix_len, int fast,
-                    unsigned long long* __restrict__ block_off /*[n_blocks+1]*/, uint8_t* __restrict__ out,
-                    uint64_t out_cap, unsigned long long* __restrict__ stats /*[8]*/,
-                    unsigned long long* __restrict__ block_adj /*[n_blocks]: slice_off[r] + block_adj[b] = where read r's slices go*/) {
-    if (threadIdx.x != 0) return;
-    unsigned long long pos = 0;
-    for (uint32_t b = 0; b < n_blocks; b++) {
-        block_off[b] = pos;
-        unsigned long long body = slice_off[block_first[b + 1]] - slice_off[block_first[b]];
-        bool empty = block_first[b + 1] == block_first[b];
-        block_adj[b] = pos + 8 + (prefix_len ? prefix_len[b] : 0) + (fast ? 4 : 0) - slice_off[block_first[b]];
-        unsigned long long extra = (prefix_len ? prefix_len[b] : 0) + ((fast && !empty) ? 4 : 0);
-        unsigned long long length = body + extra;
-        if (pos + 8 <= out_cap) {
-            uint32_t l = (uint32_t)length;
-            out[pos + 0] = (uint8_t)(l >> 24);
-            out[pos + 1] = (uint8_t)(l >> 16);
-            out[pos + 2] = (uint8_t)(l >> 8);
-            out[pos + 3] = (uint8_t)l;
-            uint64_t f = pos + 8 + (prefix_len ? prefix_len[b] : 0);
-            if (fast && !empty && f + 4 <= out_cap) {  // compressor_block.rs:95-99
-                out[f + 0] = 1;
-                out[f + 1] = 0;
-                out[f + 2] = 1;
-                out[f + 3] = 1;
-            }
+// block b's length field: its slices, the reserved prefix and the fast-mode marker (an empty block has no marker)
+__device__ __forceinline__ unsigned long long block_length(const unsigned long long* __restrict__ slice_off,
+                                                           const uint32_t* __restrict__ block_first, uint32_t b,
+                                                           const uint32_t* __restrict__ prefix_len, int fast) {
+    const unsigned long long body = slice_off[block_first[b + 1]] - slice_off[block_first[b]];
+    const bool empty = block_first[b + 1] == block_first[b];
+    return body + (prefix_len ? prefix_len[b] : 0) + ((fast && !empty) ? 4 : 0);
+}
+
+// block layout, step 1 of 3: thread per block, block_off[b] = the bytes of block b (header + length); step 2 is the
+// exclusive scan of block_off by scan_tiles_kernel, step 3 block_layout_kernel
+__global__ void block_size_kernel(const unsigned long long* __restrict__ slice_off, const uint32_t* __restrict__ block_first,
+                                  uint32_t n_blocks, const uint32_t* __restrict__ prefix_len, int fast,
+                                  unsigned long long* __restrict__ block_off /*[n_blocks+1]*/) {
+    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b < n_blocks) block_off[b] = 8 + block_length(slice_off, block_first, b, prefix_len, fast);
+}
+
+// thread per block, after the scan: block_adj, the length field and the fast-mode marker of block b at block_off[b];
+// thread 0 also leaves the container size in stats[0] (out_bytes / required_bytes).  Launch with at least one thread.
+__global__ void block_layout_kernel(const unsigned long long* __restrict__ slice_off, const uint32_t* __restrict__ block_first,
+                                    uint32_t n_blocks, const uint32_t* __restrict__ prefix_len, int fast,
+                                    const unsigned long long* __restrict__ block_off /*[n_blocks+1], scanned*/,
+                                    uint8_t* __restrict__ out, uint64_t out_cap, unsigned long long* __restrict__ stats /*[8]*/,
+                                    unsigned long long* __restrict__ block_adj /*[n_blocks]: slice_off[r] + block_adj[b] = where read r's slices go*/) {
+    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b == 0) stats[0] = block_off[n_blocks];
+    if (b >= n_blocks) return;
+    const unsigned long long pos = block_off[b];
+    const uint32_t prefix = prefix_len ? prefix_len[b] : 0;
+    block_adj[b] = pos + 8 + prefix + (fast ? 4 : 0) - slice_off[block_first[b]];
+    if (pos + 8 <= out_cap) {
+        const uint32_t l = (uint32_t)block_length(slice_off, block_first, b, prefix_len, fast);
+        out[pos + 0] = (uint8_t)(l >> 24);
+        out[pos + 1] = (uint8_t)(l >> 16);
+        out[pos + 2] = (uint8_t)(l >> 8);
+        out[pos + 3] = (uint8_t)l;
+        const uint64_t f = pos + 8 + prefix;
+        if (fast && block_first[b + 1] != block_first[b] && f + 4 <= out_cap) {  // compressor_block.rs:95-99
+            out[f + 0] = 1;
+            out[f + 1] = 0;
+            out[f + 2] = 1;
+            out[f + 3] = 1;
         }
-        pos += 8 + length;
     }
-    block_off[n_blocks] = pos;
-    stats[0] = pos;  // out_bytes / required_bytes
 }
 
 struct AssembleArgs {
@@ -941,46 +951,135 @@ struct AssembleArgs {
     const uint8_t* cand_index;  // [2][kMaxCand] candidate -> SwitchModel index (position in models[])
     uint8_t* out;
     uint64_t out_cap;
+    uint32_t lanes_log2;  // lanes per read: 1..5 (assemble_lanes_log2)
 };
 
-// copies n bytes src -> dst (any alignments) as aligned destination words built from two aligned source words
-__device__ __forceinline__ void copy_bytes_words(uint8_t* __restrict__ d, const uint8_t* __restrict__ src, uint32_t n) {
-    uint32_t head = (uint32_t)((4 - (reinterpret_cast<uintptr_t>(d) & 3)) & 3);
-    if (head > n) head = n;
-    for (uint32_t i = 0; i < head; i++) d[i] = src[i];
-    const uint32_t words = (n - head) >> 2;
-    const uint8_t* s2 = src + head;
-    const uint32_t sh = (uint32_t)(reinterpret_cast<uintptr_t>(s2) & 3);
-    const uint32_t* sw = reinterpret_cast<const uint32_t*>(s2 - sh);
-    uint32_t* dw = reinterpret_cast<uint32_t*>(d + head);
-    if (sh == 0) {
-#pragma unroll 4
-        for (uint32_t i = 0; i < words; i++) dw[i] = __ldg(sw + i);
-    } else if (words) {
-        uint32_t lo = __ldg(sw);
-#pragma unroll 4
-        for (uint32_t i = 0; i < words; i++) {
-            uint32_t hi = __ldg(sw + i + 1);  // holds at least one byte of the range: 4 * (i + 1) - sh < 4 * words + ... <= n - head
-            dw[i] = __funnelshift_r(lo, hi, 8 * sh);
-            lo = hi;
-        }
+constexpr int kAssembleBlock = 256;
+
+// the 16 bytes at address s (any alignment) from the aligned 16-byte loads that hold them; a load whose 16 bytes hold none
+// of the wanted source range [vlo, vhi) is left out (its bytes read as 0), so nothing outside that range's aligned cover
+// is touched
+__device__ __forceinline__ uint4 load_unaligned16(uintptr_t s, uintptr_t vlo, uintptr_t vhi) {
+    const uintptr_t a = s & ~(uintptr_t)15;
+    const uint32_t off = (uint32_t)(s & 15);
+    uint4 lo = make_uint4(0, 0, 0, 0), hi = make_uint4(0, 0, 0, 0);
+    if (a + 16 > vlo && a < vhi) lo = __ldg(reinterpret_cast<const uint4*>(a));
+    if (off && a + 32 > vlo && a + 16 < vhi) hi = __ldg(reinterpret_cast<const uint4*>(a + 16));
+    // words w0 .. w7 = lo | hi; drop off / 4 words, then funnel-shift by the byte rest
+    uint32_t w0 = lo.x, w1 = lo.y, w2 = lo.z, w3 = lo.w, w4 = hi.x, w5 = hi.y, w6 = hi.z, w7 = hi.w;
+    if (off & 8) {
+        w0 = w2, w1 = w3, w2 = w4, w3 = w5, w4 = w6, w5 = w7;
     }
-    for (uint32_t i = head + 4 * words; i < n; i++) d[i] = src[i];
+    if (off & 4) {
+        w0 = w1, w1 = w2, w2 = w3, w3 = w4, w4 = w5;
+    }
+    const uint32_t sh = 8 * (off & 3);
+    return make_uint4(__funnelshift_r(w0, w1, sh), __funnelshift_r(w1, w2, sh), __funnelshift_r(w2, w3, sh),
+                      __funnelshift_r(w3, w4, sh));
 }
 
-// one thread per read: slice headers + payload copy from the scratch slot to its final place.  The threads of a warp
-// own neighbouring reads, i.e. neighbouring scratch slots and neighbouring destinations.
-__global__ void __launch_bounds__(128)
+// bytes [k0, k1) of the 16-byte destination chunk at d (the bytes around them belong to somebody else)
+__device__ __forceinline__ void store_bytes16(uint8_t* d, uint4 v, uint32_t k0, uint32_t k1) {
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (uint32_t k = 0; k < 16; k++)
+        if (k >= k0 && k < k1) d[k] = (uint8_t)(w[k >> 2] >> (8 * (k & 3)));
+}
+
+// destination chunk c of a read (assemble_kernel): its address, its bytes [k0, k1) to write and their values
+struct AssembleChunk {
+    uintptr_t a;
+    uint4 v;
+    uint32_t k0, k1;
+};
+__device__ __forceinline__ AssembleChunk assemble_chunk(uint32_t c, uint32_t n_chunks, uintptr_t c0, uintptr_t d, uintptr_t e,
+                                                        uintptr_t s, uintptr_t pe, bool fits, bool prev_fits) {
+    AssembleChunk x;
+    x.a = c0 + 16ull * c;
+    x.v = make_uint4(0, 0, 0, 0);
+    x.k0 = x.k1 = 0;
+    if (c >= n_chunks) return x;
+    const uintptr_t a = x.a;
+    // chunk bytes [0, split) belong to the previous read, [split, k_end) to this one
+    const uint32_t split = a < d ? (uint32_t)(d - a) : 0u;
+    const uint32_t k_end = a + 16 <= e ? 16u : (uint32_t)(e - a);
+    x.k0 = (split && prev_fits) ? 0u : split;
+    x.k1 = fits ? k_end : split;
+    if (x.k1 > split) x.v = load_unaligned16(s + (a - d), s + (a + split - d), s + (a + k_end - d));  // chunk byte k <- s + (a + k - d)
+    if (split && x.k0 == 0) {
+        const uint4 p = load_unaligned16(pe - split, pe - split, pe);
+        // bytes below split from p
+        const uint32_t m0 = split >= 4 ? 0xffffffffu : (1u << (8 * split)) - 1;
+        const uint32_t m1 = split >= 8 ? 0xffffffffu : split <= 4 ? 0u : (1u << (8 * (split - 4))) - 1;
+        const uint32_t m2 = split >= 12 ? 0xffffffffu : split <= 8 ? 0u : (1u << (8 * (split - 8))) - 1;
+        const uint32_t m3 = split <= 12 ? 0u : (1u << (8 * (split - 12))) - 1;
+        x.v.x = (p.x & m0) | (x.v.x & ~m0);
+        x.v.y = (p.y & m1) | (x.v.y & ~m1);
+        x.v.z = (p.z & m2) | (x.v.z & ~m2);
+        x.v.w = (p.w & m3) | (x.v.w & ~m3);
+    }
+    return x;
+}
+
+// Lanes per read for assemble_kernel: two passes of two 16-byte chunks per lane for a read of the call's mean length at
+// about one byte of slices per symbol, 2 lanes (reads of up to ~100 symbols) to 32 (a warp per read, which loops over
+// long reads).  Few lanes per read keep many reads -- many independent loads -- in each warp (on hiseq100, 8 lanes per
+// read: 3.3 ms, 4: 2.9 ms, 2: 2.2 ms).
+inline uint32_t assemble_lanes_log2(uint64_t n_symbols, uint64_t n_reads) {
+    const uint64_t mean = n_reads ? n_symbols / n_reads : 0;
+    const uint64_t chunks = (mean + 9 + 15) / 16 + 1;
+    uint32_t l2 = 1;
+    while (l2 < 5 && (4ull << l2) < chunks) l2++;
+    return l2;
+}
+
+// Copies the reads' finished slices from their scratch slots into the container.  Within a block the slices of
+// consecutive reads lie back to back, so the container body is cut into aligned 16-byte destination chunks, and a chunk
+// belongs to the read that holds its LAST byte: its leading bytes, when it has any before the read's first byte, are the
+// last bytes of the read before (whose slot ends at 4*read_off[r] + kSlotExtra*r; every read has at least 17 bytes of
+// slices, so no chunk reaches two reads back).  A group of 2^lanes_log2 lanes owns a read and moves its chunks as whole
+// 16-byte stores, two per lane and pass, each built by funnel shifts from two aligned 16-byte loads per source read; consecutive lanes take
+// consecutive chunks, so a warp instruction covers a few hundred contiguous destination bytes instead of 32 scattered
+// words.  Bytes are written one by one only where a chunk holds bytes that are not slices of the block: the first chunk
+// of a block's first read, the tail of its last read (the last read also owns the chunk that holds its last byte), and
+// the reads that do not fit the capacity.  A read is written completely or not at all: never at or past out_cap
+// (IDN_E_NOSPACE is reported by the host from stats).
+__global__ void __launch_bounds__(kAssembleBlock, 6)
 assemble_kernel(AssembleArgs A) {
-    uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint64_t t = (uint64_t)blockIdx.x * kAssembleBlock + threadIdx.x;
+    const uint64_t r = t >> A.lanes_log2;
+    const uint32_t lanes = 1u << A.lanes_log2, j = (uint32_t)t & (lanes - 1);
     if (r >= A.n_reads) return;
-    const unsigned long long dst = A.slice_off[r] + A.block_adj[A.read_block[r]];
+    const uint32_t blk = A.read_block[r];
+    const bool first = r == 0 || A.read_block[r - 1] != blk;
+    const bool last = r + 1 == A.n_reads || A.read_block[r + 1] != blk;
+    const unsigned long long dst = A.slice_off[r] + A.block_adj[blk];
     uint32_t nsw = 0;
     if (A.switched) nsw = A.switched[r] + A.switched[A.n_reads + r];
     const uint32_t total = 2u * nsw + 9u + A.pay_len[r];  // the encoder left the read's slices complete in its scratch slot
-    if (dst + total > A.out_cap) return;  // IDN_E_NOSPACE is reported by the host from stats
-    const uint8_t* src = A.scratch + 4ull * A.read_off[r + 1] + kSlotExtra * (r + 1) - total;
-    copy_bytes_words(A.out + dst, src, total);
+    const bool fits = dst + total <= A.out_cap;
+    const bool prev_fits = !first && dst <= A.out_cap;  // the read before ends at dst
+    if (!fits && !prev_fits) return;
+    const uintptr_t out = reinterpret_cast<uintptr_t>(A.out);
+    const uintptr_t scr = reinterpret_cast<uintptr_t>(A.scratch);
+    const uintptr_t d = out + dst, e = d + total;                                        // this read's destination bytes
+    const uintptr_t s = scr + 4ull * A.read_off[r + 1] + kSlotExtra * (r + 1) - total;  // and their source
+    const uintptr_t pe = scr + 4ull * A.read_off[r] + kSlotExtra * r;                   // end of the previous read's source
+    const uintptr_t c0 = d & ~(uintptr_t)15;
+    const uint32_t n_chunks = (uint32_t)(((e & ~(uintptr_t)15) - c0) >> 4) + ((last && (e & 15)) ? 1u : 0u);
+    // two chunks per lane and pass: both chunks' loads are in flight before the first store
+#pragma unroll 1
+    for (uint32_t c = j; c < n_chunks; c += 2 * lanes) {
+        AssembleChunk x[2];
+#pragma unroll
+        for (int u = 0; u < 2; u++) x[u] = assemble_chunk(c + u * lanes, n_chunks, c0, d, e, s, pe, fits, prev_fits);
+#pragma unroll
+        for (int u = 0; u < 2; u++) {
+            uint8_t* dp = reinterpret_cast<uint8_t*>(x[u].a);
+            if (x[u].k0 == 0 && x[u].k1 == 16) *reinterpret_cast<uint4*>(dp) = x[u].v;
+            else if (x[u].k1 > x[u].k0) store_bytes16(dp, x[u].v, x[u].k0, x[u].k1);
+        }
+    }
 }
 
 // read -> block map (one thread per block fills its range; blocks are large, so use a grid-stride loop)
