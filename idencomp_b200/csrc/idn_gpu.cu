@@ -274,7 +274,9 @@ struct SmallParams {
     uint32_t native_split;   // native decode: some block of the call cuts long reads into pieces
     uint32_t pad[2];
     unsigned long long stats[8];
-    int32_t status[4];
+    // decode side: [0] code, [1] block, [2] reads needed (NoSpace), [3] first block with a checksum mismatch, [4..5] first
+    // block failure of the walk / lane table as one u64 key (fail_key, idn_kernels.cuh), [6] first block with a stream error
+    int32_t status[8];
 };
 
 }  // namespace
@@ -1470,6 +1472,8 @@ static void fill_decode_params(idn_gpu_ctx* ctx, SmallParams* sp, const idn_mode
         sp->model_type[i] = (uint8_t)ctx->slots[models[i]].dev.type;
     }
     sp->status[1] = -1;
+    sp->status[4] = sp->status[5] = -1;  // fail_key: none
+    sp->status[6] = 0x7fffffff;  // no stream error
 }
 
 static int32_t decompress_native_dev(idn_gpu_ctx* ctx, const uint8_t* blocks, const unsigned long long* boff,
@@ -1503,7 +1507,7 @@ static int32_t decompress_native_dev(idn_gpu_ctx* ctx, const uint8_t* blocks, co
     LAUNCHED("scan_tiles");
     scan_tiles_kernel<<<1, kScanBlock, 0, st>>>(bc.slots, n_blocks);
     LAUNCHED("scan_tiles");
-    index_check_kernel<<<(n_blocks + 1 + 255) / 256, 256, 0, st>>>(bc.reads, bc.syms, n_blocks, out_reads_cap, out_symbols_cap,
+    index_check_kernel<<<(n_blocks + 1 + 255) / 256, 256, 0, st>>>(bc.reads, bc.syms, bc.slots, n_blocks, out_reads_cap, out_symbols_cap,
                                                                  block_first, dsp->status);
     LAUNCHED("index_check");
     native_fill_kernel<<<n_blocks + 1, kScanBlock, 0, st>>>(blocks, hdr, n_blocks, bc.reads, bc.syms, bc.slots, roff, ix,
@@ -1523,6 +1527,9 @@ static int32_t decompress_native_dev(idn_gpu_ctx* ctx, const uint8_t* blocks, co
         da.quals_out = quals_out;
         da.out_dq = (long long)(quals_out - acids_out);
         da.err = &dsp->err;
+        da.err_block = dsp->status + 6;
+        da.blk_lane_base = bc.slots;
+        da.n_blocks = n_blocks;
         da.part_crc = nullptr;
         da.part_len = nullptr;
         da.crc_tab = da.xpow = nullptr;
@@ -1640,7 +1647,7 @@ extern "C" int32_t idn_gpu_decompress_blocks_dev(idn_gpu_ctx* ctx, const uint8_t
         roff = ctx->w_sliceoff.as<unsigned long long>();
     }
     // capacity check on the device; on failure the later kernels are no-ops
-    index_check_kernel<<<(n_blocks + 1 + 255) / 256, 256, 0, st>>>(bc.reads, bc.syms, n_blocks, out_reads_cap, out_symbols_cap,
+    index_check_kernel<<<(n_blocks + 1 + 255) / 256, 256, 0, st>>>(bc.reads, bc.syms, bc.slots, n_blocks, out_reads_cap, out_symbols_cap,
                                                                  block_first, dsp->status);
     LAUNCHED("index_check");
     DecodeArgs da;
@@ -1660,6 +1667,7 @@ extern "C" int32_t idn_gpu_decompress_blocks_dev(idn_gpu_ctx* ctx, const uint8_t
     da.read_off_out = roff;
     da.read_status = nullptr;
     da.err = &dsp->err;
+    da.err_block = dsp->status + 6;
     da.part_crc = nullptr;
     da.part_len = nullptr;
     da.crc_tab = da.xpow = nullptr;
@@ -1807,12 +1815,16 @@ extern "C" int32_t idn_gpu_index_blocks(idn_gpu_ctx* ctx, const uint8_t* blocks,
         return fail(ctx, IDN_E_UNSUPPORTED, "unknown mode %d", mode);
     }
     std::vector<unsigned long long> hr(n_blocks + 1), hsym(n_blocks + 1);
-    int32_t hst[4];
+    int32_t hst[8];
     BlockCounters bc = carve_counters(ctx->w_blk.p, n_blocks);
     CU(cudaMemcpyAsync(hr.data(), bc.reads, ((size_t)n_blocks + 1) * 8, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(hsym.data(), bc.syms, ((size_t)n_blocks + 1) * 8, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(hst, dsp->status, sizeof hst, cudaMemcpyDeviceToHost, st));
     CU(sync_stream(ctx, st));
+    if (hst[0] == 0 && hst[5] != -1) {  // the first block whose walk / lane table failed (status[4..5] = block << 32 | code)
+        hst[0] = hst[4];
+        hst[1] = hst[5];
+    }
     if (hst[0]) return status_to_error(ctx, hst);
     totals->n_reads = hr[n_blocks];
     totals->n_symbols = hsym[n_blocks];
@@ -2061,6 +2073,7 @@ extern "C" int32_t idn_gpu_decompress_reads(idn_gpu_ctx* ctx, const uint8_t* pay
     da.read_off_out = nullptr;
     da.read_status = ctx->s_idx.as<uint32_t>();
     da.err = &dsp->err;
+    da.err_block = nullptr;
     da.part_crc = nullptr;
     da.part_len = nullptr;
     da.crc_tab = da.xpow = nullptr;

@@ -1447,6 +1447,18 @@ __device__ __forceinline__ uint32_t load_u32be(const uint8_t* p) {
     return ((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | p[3];
 }
 
+// Decode-side errors are reported for the first failing block in file order, whichever thread block gets there first.
+// A block whose slices (compat) or lane table (native) are malformed records (block << 32 | code) with atomicMin in
+// status[4..5] (~0 = none); index_check_kernel then cuts the call at that block, so the blocks in front of it are still
+// decoded and checked, and finish_decode_kernel reports the lowest block among that failure, the checksum mismatches
+// (status[3]) and the rANS stream errors (status[6]).
+__device__ __forceinline__ unsigned long long fail_key(const int32_t* status) {
+    return *reinterpret_cast<const volatile unsigned long long*>(status + 4);
+}
+__device__ __forceinline__ void fail_block(int32_t* status, uint32_t b, int32_t code) {
+    atomicMin(reinterpret_cast<unsigned long long*>(status + 4), ((unsigned long long)b << 32) | (uint32_t)code);
+}
+
 struct ReadIndexDev {  // per-read index, strided by block (see above) or dense (idn_gpu_decompress_reads)
     unsigned long long* pay_off;  // absolute offset of the rANS payload in `payload`
     uint32_t* pay_len;
@@ -1512,7 +1524,7 @@ walk_kernel(const uint8_t* __restrict__ blocks, const unsigned long long* __rest
             const uint32_t* __restrict__ block_len, uint32_t n_blocks, unsigned long long blocks_bytes,
             const uint8_t* __restrict__ model_type /*[n_models] by container index*/, uint32_t n_models,
             const unsigned long long* __restrict__ slot_base, ReadIndexDev ix, unsigned long long* __restrict__ blk_reads,
-            unsigned long long* __restrict__ blk_syms, int32_t* __restrict__ status /*[2]: code, block*/,
+            unsigned long long* __restrict__ blk_syms, int32_t* __restrict__ status /*SmallParams::status*/,
             const uint8_t* __restrict__ done /*blocks walk_fast_kernel has indexed, or nullptr*/) {
     __shared__ __align__(16) uint8_t tiles[2][kWalkTile + 32];
     __shared__ uint16_t plist[kWalkMaxEnt];  // tile offsets of the slice headers found in the current tile
@@ -1666,10 +1678,7 @@ walk_kernel(const uint8_t* __restrict__ blocks, const unsigned long long* __rest
     if (lane == 0) {
         blk_reads[b] = n_reads;
         blk_syms[b] = n_syms;
-        if (st != 0) {
-            int old = atomicCAS(&status[0], 0, st);
-            if (old == 0) status[1] = (int32_t)b;
-        }
+        if (st != 0) fail_block(status, b, st);
     }
 }
 
@@ -1909,17 +1918,32 @@ walk_fast_kernel(const uint8_t* __restrict__ blocks, const unsigned long long* _
 }
 
 // totals against the caller's capacities + u32 block_first for the CRC kernels; on failure every later kernel of the
-// call is a no-op
+// call is a no-op.  A block f that failed its walk / lane table cuts the call: the scans of reads, symbols and index slots
+// (lanes) stop at f, so the decoders and the CRC check see blocks [0, f) only.
 __global__ void __launch_bounds__(256)
-index_check_kernel(const unsigned long long* __restrict__ blk_reads, const unsigned long long* __restrict__ blk_syms,
-                   uint32_t n_blocks, uint64_t reads_cap, uint64_t syms_cap, uint32_t* __restrict__ block_first,
-                   int32_t* __restrict__ status) {
+index_check_kernel(unsigned long long* __restrict__ blk_reads, unsigned long long* __restrict__ blk_syms,
+                   unsigned long long* __restrict__ blk_slots, uint32_t n_blocks, uint64_t reads_cap, uint64_t syms_cap,
+                   uint32_t* __restrict__ block_first, int32_t* __restrict__ status) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i <= n_blocks && block_first) block_first[i] = (uint32_t)blk_reads[i];
+    const unsigned long long key = fail_key(status);
+    const uint32_t f = key == ~0ull ? n_blocks : (uint32_t)(key >> 32);  // (entry f itself is never written here)
+    if (i <= n_blocks) {
+        if (i > f) {
+            blk_reads[i] = blk_reads[f];
+            blk_syms[i] = blk_syms[f];
+            blk_slots[i] = blk_slots[f];
+        }
+        if (block_first) block_first[i] = (uint32_t)blk_reads[i < f ? i : f];
+    }
     if (i != 0) return;
     status[3] = 0x7fffffff;  // first block with a checksum mismatch
     if (status[0] != 0) return;
-    if (blk_reads[n_blocks] > reads_cap || blk_syms[n_blocks] > syms_cap) {
+    if (blk_reads[f] > reads_cap || blk_syms[f] > syms_cap) {
+        if (f < n_blocks) {  // the blocks in front of the failing one do not fit: its failure stands
+            status[0] = (int32_t)(uint32_t)key;
+            status[1] = (int32_t)f;
+            return;
+        }
         status[0] = 11;  // IDN_E_NOSPACE
         status[1] = -1;
         status[2] = (int32_t)(blk_reads[n_blocks] > 0x7fffffffull ? 0x7fffffff : blk_reads[n_blocks]);
@@ -1957,6 +1981,7 @@ struct DecodeArgs {
     unsigned long long* read_off_out;       // optional [n_reads+1]: absolute symbol offset of every read
     uint32_t* read_status;  // optional
     uint32_t* err;
+    int32_t* err_block;     // optional (block-strided index): atomicMin of the block of a read whose stream fails
     // optional: CRC-32 partial of every decoded read (acids | quals), the input of crc_verify_kernel, computed while the
     // symbols are in registers instead of by a second pass over the output (K7 fused into K5)
     uint32_t* part_crc;
@@ -2223,15 +2248,21 @@ __device__ __forceinline__ void decode_read_body(const ModelDev& ma, const Model
     }
 }
 
+// largest b < n_blocks with base[b] <= v (base: an exclusive scan per block)
+__device__ __forceinline__ uint32_t block_of(const unsigned long long* __restrict__ base, uint32_t n_blocks, unsigned long long v) {
+    uint32_t lo = 0, hi = n_blocks;
+    while (hi - lo > 1) {
+        uint32_t mid = (lo + hi) >> 1;
+        if (__ldg(base + mid) <= v) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
 // block and index slot of read r of a block-strided index; false past the last read
 __device__ __forceinline__ bool decode_locate(const DecodeArgs& A, uint64_t r, unsigned long long& slot, unsigned long long& sym_base) {
     const unsigned long long R = A.blk_read_base[A.n_blocks];
     if (r >= R) return false;
-    uint32_t lo = 0, hi = A.n_blocks;  // largest b with blk_read_base[b] <= r
-    while (hi - lo > 1) {
-        uint32_t mid = (lo + hi) >> 1;
-        if (__ldg(A.blk_read_base + mid) <= r) lo = mid; else hi = mid;
-    }
+    const uint32_t lo = block_of(A.blk_read_base, A.n_blocks, r);
     slot = A.slot_base[lo] + (r - A.blk_read_base[lo]);
     sym_base = A.blk_sym_base[lo];
     return true;
@@ -2265,7 +2296,10 @@ __device__ __forceinline__ void decode_one(const DecodeArgs& A, const ModelDev& 
     uint32_t st = D.st;
     if (!(st & 1) && !D.clean_end(plen)) st |= 2;
     if (A.read_status) A.read_status[r] = st;
-    if (st) atomicOr(A.err, 1u);
+    if (st) {
+        atomicOr(A.err, 1u);
+        if (A.err_block) atomicMin(A.err_block, (int32_t)block_of(A.blk_read_base, A.n_blocks, r));
+    }
     if (A.part_crc) {  // crc(acids | quals) of this read, as crc_read_kernel would compute it
         const CrcPair p = crc_concat(CrcPair{~C.ca, len}, CrcPair{~C.cq, len}, s_xpow);
         A.part_crc[r] = len ? p.crc : 0u;
@@ -2328,8 +2362,29 @@ __global__ void finish_decode_kernel(const int32_t* __restrict__ status, const u
     int32_t code = status[0];
     uint64_t R = *n_reads_total;
     int32_t blk = status[1];
-    if (code == 0 && (*err & 1u)) code = 3;  // a payload ran out: IDN_E_SERIALIZE
-    if (code == 6) blk = status[3];
+    if (code != 11 && code != 12) {
+        // block failures: the lowest block wins; within one block a malformed walk / lane table before a checksum mismatch
+        // before a stream that runs out or does not end cleanly (IDN_E_SERIALIZE)
+        unsigned long long best = ~0ull;
+        int32_t best_code = 0;
+        auto take = [&](unsigned long long b, unsigned rank, int32_t c) {
+            const unsigned long long k = b << 2 | rank;
+            if (k < best) {
+                best = k;
+                best_code = c;
+            }
+        };
+        const unsigned long long key = fail_key(status);
+        if (key != ~0ull) take(key >> 32, 0, (int32_t)(uint32_t)key);
+        if (code == 6) take((uint32_t)status[3], 1, 6);
+        if (status[6] != 0x7fffffff) take((uint32_t)status[6], 2, 3);
+        if (best_code) {
+            code = best_code;
+            blk = (int32_t)(best >> 2);
+        } else if (*err & 1u) {
+            code = 3;  // a payload ran out: IDN_E_SERIALIZE
+        }
+    }
     status_dev[0] = code;
     status_dev[1] = blk;
     status_dev[2] = code == 11 ? status[2] : (int32_t)(R > 0x7fffffffull ? 0x7fffffff : R);

@@ -505,10 +505,7 @@ native_hdr_kernel(const uint8_t* __restrict__ blocks, const unsigned long long* 
         blk_reads[b] = st == 0 ? h.n_reads : 0;
         blk_syms[b] = st == 0 ? syms : 0;
         blk_lanes[b] = st == 0 ? h.n_lanes : 0;
-        if (st != 0) {
-            int old = atomicCAS(&status[0], 0, st);
-            if (old == 0) status[1] = (int32_t)b;
-        }
+        if (st != 0) fail_block(status, b, st);
     }
 }
 
@@ -533,11 +530,17 @@ native_fill_kernel(const uint8_t* __restrict__ blocks, const NativeBlockHdr* __r
     __shared__ unsigned long long total;
     __shared__ int lane_mismatch;
     __shared__ int32_t s_status;
+    __shared__ uint32_t s_stop;
     const uint32_t b = blockIdx.x;
-    // other CTAs of this launch may set status[0] while this one runs: every thread must take the same exit (barriers follow)
-    if (threadIdx.x == 0) s_status = status[0];
+    // other CTAs of this launch may set status[0] / the failure key while this one runs: every thread must take the same
+    // exit (barriers follow).  s_stop: the first block that failed its header; the call stops in front of it.
+    if (threadIdx.x == 0) {
+        s_status = status[0];
+        s_stop = (uint32_t)(fail_key(status) >> 32);
+    }
     __syncthreads();
     if (s_status != 0) return;
+    if (b < n_blocks && b >= s_stop) return;
     if (blk_lane_base[n_blocks] + 1 > ix.cap) {  // more lanes than the index holds: refuse (uniform over the launch)
         if (b == 0 && threadIdx.x == 0) {
             int old = atomicCAS(&status[0], 0, 11);  // IDN_E_NOSPACE
@@ -644,9 +647,9 @@ native_fill_kernel(const uint8_t* __restrict__ blocks, const NativeBlockHdr* __r
         __syncthreads();
     }
     __syncthreads();
-    if (threadIdx.x == 0 && lane_mismatch) {
-        int old = atomicCAS(&status[0], 0, 3);  // the lane table does not match the partition of the lengths
-        if (old == 0) status[1] = (int32_t)b;
+    if (threadIdx.x == 0 && lane_mismatch) {  // the lane table does not match the partition of the lengths
+        fail_block(status, b, 3);
+        atomicCAS(&status[0], 0, 3);  // the lanes of this block are not indexed: no lane of the call may decode
     }
 }
 
@@ -664,6 +667,9 @@ struct DecodeLaneArgs {
     uint8_t* quals_out;
     long long out_dq;  // quals_out - acids_out
     uint32_t* err;
+    int32_t* err_block;                       // atomicMin of the block of a lane whose stream fails
+    const unsigned long long* blk_lane_base;  // [n_blocks + 1] exclusive scan of the lanes per block
+    uint32_t n_blocks;
     // optional: per-read CRC-32 partials (acids | quals) for crc_verify_kernel, as in DecodeArgs
     uint32_t* part_crc;
     unsigned long long* part_len;
@@ -710,7 +716,10 @@ __device__ __forceinline__ void decode_lane_one(const DecodeLaneArgs& A, const M
     O.flush();
     const uint32_t plen = A.ix.pay_len[l] - lead;
     D.finish(A.payload + A.ix.pay_off[l], lead, plen);
-    if (bad || (D.st & 1) || !D.clean_end(plen)) atomicOr(A.err, 1u);
+    if (bad || (D.st & 1) || !D.clean_end(plen)) {
+        atomicOr(A.err, 1u);
+        atomicMin(A.err_block, (int32_t)block_of(A.blk_lane_base, A.n_blocks, l64));
+    }
 }
 
 template <bool kUniform, class P>

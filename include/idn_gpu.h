@@ -172,6 +172,12 @@ uint64_t idn_gpu_compress_bound(uint64_t n_reads, uint64_t n_symbols, uint32_t n
  * the block has no names).  A Sequence slice (or native lane) whose rANS stream runs out early, or does not end with
  * both states back at their initial value and every payload byte consumed, fails the call with IDN_E_SERIALIZE in both
  * container modes, with or without a CRC to compare against.
+ * A failing call reports the first failing block in file order (bad_block / status_dev[1]; -1 only for errors of the
+ * whole call such as IDN_E_NOSPACE): the blocks in front of a malformed one are still decoded and checked, so a
+ * checksum mismatch or a garbled stream there is reported instead; within one block malformed slices come before a
+ * checksum mismatch before a garbled stream.  The report does not depend on idn_gpu_set_walk, on
+ * idn_gpu_set_pipeline_blocks or on the entry point.  (A native lane table that does not match its read lengths stops
+ * the call where it is found: the blocks in front of it are not checked.)
  * Two-step use: idn_gpu_index_blocks returns the read count / symbol count so the caller can size the
  * outputs, then idn_gpu_decompress_blocks fills them.  The index call leaves the container bytes on the device: a
  * decode call (idn_gpu_decompress_blocks, idn_gpu_decompress_to_fastq) that follows it on the same context with the
